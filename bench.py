@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Mrays/s (all ray types) and ms/frame of the Whitted hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A step = one frame of the workload (default: BASELINE.json configs[3], out/water_bunny_tex.txt
 + `shadow soft` at 3840x2160 — the configuration the north-star metric is quoted on).
@@ -13,6 +13,8 @@ render + image D2H inside the timed region).  `--impl reference` times the UNMOD
 reference (oracle/_ref, single-threaded by construction) on a bounded pixel sample of the
 same frame; beside its value the line carries `all_cores`: the same sample traced by one
 independent reference process per host core (what the whole host could do; not the reference's mode).
+`--dump-outputs DIR` writes the frame and ray counts of the last timed step as .npy files (dump_outputs): the inputs
+are the same from run to run, so two builds can be compared output for output.
 """
 from __future__ import annotations
 
@@ -62,6 +64,13 @@ ALGO_BYTES = {
     "soft_lists": 32.0 + 8.0 + 4.0 * 25.0, # per request: request read, reference + list written
     "shadow_directional": 36.0,
 }
+
+
+# --dump-outputs: at most this many bytes of .npy data; a larger frame is dumped as a fixed, seeded pixel sample
+DUMP_BUDGET_BYTES = 64 << 20
+DUMP_SAMPLE_PIXELS = 1 << 21
+DUMP_SEED = 0
+DUMP_COUNTS = ("closest_rays", "shadow_rays", "shadow_requests")     # + rays_per_depth
 
 
 def flops_per_ray(workload):
@@ -286,8 +295,28 @@ KERNEL_NAMES = {"shadow_soft": "k_soft_list_rays", "soft_lists": "k_soft_lists",
                 "shade": "k_shade", "combine": "k_combine_resolve", "soft_filter": "k_soft_filter"}
 
 
-def measure_workload(workload, steps, warmup, dist_env, cpu_seconds, want_clocks):
-    """Benchmarks one workload on this rank (all ranks call it together).  Returns the JSON-line dict on rank 0."""
+def dump_outputs(out_dir, image, counts):
+    """--dump-outputs: what the timed path returned in its last step, as .npy files in `out_dir`.  image.npy is the
+    (H, W, 3) frame as float32 or, when that would exceed half of DUMP_BUDGET_BYTES, the pixels at DUMP_SAMPLE_PIXELS
+    fixed, seeded positions ((N, 3) float32, positions y * W + x in image_pixel_index.npy); every entry of `counts`
+    (the frame's ray counts) goes to <name>.npy as float64."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    h, w, _ = image.shape
+    if h * w * 3 * 4 > DUMP_BUDGET_BYTES // 2:
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, DUMP_SAMPLE_PIXELS, replace=False))
+        np.save(out / "image.npy", image.reshape(-1, 3)[idx].astype(np.float32))
+        np.save(out / "image_pixel_index.npy", idx.astype(np.float64))
+    else:
+        np.save(out / "image.npy", image.astype(np.float32))
+    for name, v in counts.items():
+        np.save(out / f"{name}.npy", np.asarray(v, dtype=np.float64))
+
+
+def measure_workload(workload, steps, warmup, dist_env, cpu_seconds, want_clocks, dump_dir=None):
+    """Benchmarks one workload on this rank (all ranks call it together).  Returns the JSON-line dict on rank 0.
+    With `dump_dir`, rank 0 also writes the frame and ray counts of the last timed step there (dump_outputs)."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -346,10 +375,20 @@ def measure_workload(workload, steps, warmup, dist_env, cpu_seconds, want_clocks
         ev[k][0].record()
         dr.frame()
         ev[k][1].record()
-        dr.finish()
+        last = dr.finish()
     dr.render_done = None
     barrier()
     t_wall1 = time.time()
+    dump = None
+    if dump_dir is not None:                    # the last timed step's frame and counts, before later passes overwrite them
+        cnt = torch.tensor([last[k] for k in DUMP_COUNTS] + last["rays_per_depth"], dtype=torch.int64, device="cuda")
+        if world > 1:
+            dist.all_reduce(cnt)
+        cnt = cnt.tolist()
+        if rank == 0:
+            counts = dict(zip(DUMP_COUNTS, cnt))
+            counts["rays_per_depth"] = cnt[len(DUMP_COUNTS):]
+            dump = (dr.image.cpu().numpy(), counts)
     launches = ctx.launches - launches0
     ms_local = sum(a.elapsed_time(b) for a, b, _ in ev)
     render_local = sum(a.elapsed_time(c) for a, _, c in ev) / steps      # this rank's tiles only, no gather
@@ -518,6 +557,8 @@ def measure_workload(workload, steps, warmup, dist_env, cpu_seconds, want_clocks
     dr.close()
     del flush
     torch.cuda.empty_cache()
+    if dump is not None:
+        dump_outputs(dump_dir, *dump)
     return line
 
 
@@ -539,7 +580,7 @@ def run_cuda_arm(args):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
     env = (world, rank, local)
     cpu_s = 0.0 if args.no_cpu_baseline else args.cpu_seconds
-    line = measure_workload(args.workload, args.steps, args.warmup, env, cpu_s, True)
+    line = measure_workload(args.workload, args.steps, args.warmup, env, cpu_s, True, args.dump_outputs)
     # The other BASELINE.json configs and the section-8 f4 workloads ride along in the same line (N = 1 only, fewer
     # steps, a smaller CPU sample each) so that the driver's record carries all of them.
     if world == 1 and args.workload == DEFAULT_WORKLOAD and not args.no_per_config:
@@ -622,9 +663,15 @@ def main():
     ap.add_argument("--per-config-cpu-seconds", type=float, default=4.0)
     ap.add_argument("--ref-step-seconds", type=float, default=None,
                     help="--impl reference: CPU seconds per step's pixel sample (default: 150 s / (steps + warmup), 1..10 s)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps of --workload, write its last step's frame and ray counts to "
+                         "DIR/<name>.npy (float32 / float64, at most 64 MiB: a larger frame as a fixed, seeded pixel "
+                         "sample); the per_config runs that follow the default workload are not dumped")
     args = ap.parse_args()
     if args.steps < 1:
         raise SystemExit("--steps must be >= 1")
+    if args.dump_outputs is not None and args.impl == "reference":
+        raise SystemExit("--dump-outputs writes what the CUDA path computed; it does not apply to --impl reference")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_cuda_arm(args)

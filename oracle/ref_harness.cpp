@@ -1,5 +1,6 @@
 // ref_harness.cpp — TEST INFRASTRUCTURE.  Thin C ABI around the UNMODIFIED
-// reference headers, compiled from where they lie (-I/root/reference/include)
+// reference headers, compiled from where they lie (-I$(REF)/include, REF = the
+// reference's source tree, oracle/Makefile)
 // into oracle/_ref/libwhitted_ref.so by oracle/Makefile.  No reference source is
 // copied into this repository; this file only *calls* the reference:
 //   PPMGenerator(path) + main()'s bunny load     src/main.cpp:20-56

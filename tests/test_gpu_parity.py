@@ -451,12 +451,12 @@ def test_drop_in_executable(workdir):
 
 def test_reference_renderer_with_cuda_strategy(workdir):
     """INTEGRATION.md level A: the reference's UNMODIFIED main.cpp / Renderer with
-    integration/CudaStrategy.hpp plugged in at IIntersectStrategy (built in the container by
-    `make -C oracle ref_cuda`) — every UpdateInter / getShadowCoeffi call of the reference's own
+    integration/CudaStrategy.hpp plugged in at IIntersectStrategy (built by build() with
+    WRT_REFERENCE_DIR set, through `make -C oracle ref_cuda`) — every UpdateInter / getShadowCoeffi call of the reference's own
     recursion runs on the GPU.  Its PPM must equal the stock reference executable's."""
     strat, stock = ob.REF_EXE.parent / "whitted_ref_cuda_strategy", ob.REF_EXE
     if not (strat.exists() and stock.exists()):
-        pytest.skip("oracle/_ref executables not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref executables not built (build() with WRT_REFERENCE_DIR set)")
     fixtures.write_config(workdir, "plug", fixtures.bunny_shadow_config(64, 48))
     out = {}
     for name, exe in (("stock", stock), ("cuda", strat)):
