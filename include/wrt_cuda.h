@@ -51,6 +51,14 @@ int  wrt_create(int device, WrtContext** out);
 void wrt_destroy(WrtContext* ctx);
 const char* wrt_last_error(void);
 
+/* Uploads the scene and builds the walked tree on the device (PLOC).  The traversal stack holds 90 rows:
+ * max(reference tree depth, walked depth, 3 * ceil(walked depth / 2)) + 2 <= 90, i.e. the caller's (reference) tree
+ * may be 88 levels deep and the walked tree 58.  When PLOC's tree is deeper (fans of triangles sharing a vertex,
+ * slivers, boxes of very mixed sizes), the walked tree is rebuilt with the host's binned SAH instead; the scene is
+ * refused only if that tree or the reference's does not fit either.  Results do not depend on which tree is walked.
+ * Hard-shadow coefficients are the reference's bit for bit up to 12 translucent blockers on one ray; beyond, the
+ * product is taken in visit order (within a few ulp: the tests allow k ulp for k blockers).  WRT_VERBOSE=1 prints
+ * the builder used and the stack rows. */
 int wrt_upload_scene(WrtContext* ctx, const WrtSceneDesc* scene);
 int wrt_set_camera(WrtContext* ctx, const WrtCamera* cam);
 

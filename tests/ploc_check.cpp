@@ -3,6 +3,8 @@
 //   every primitive in exactly one leaf, leaf boxes == the reference's per-primitive boxes, every inner box the exact
 //   union of its children (and likewise the dilated boxes), sibling pairs adjacent with the parent's link pointing at
 //   them, record count 2n, depth as reported, surface-area cost close to the host's binned-SAH build.
+// Also prints the depths of the host's binned-SAH tree and of the scene's own (reference) tree: the traversal stack is
+// sized from all three (wrt_upload_scene).
 // usage: ploc_check <config> <obj|""> <asset_dir>      prints one JSON line
 #include <algorithm>
 #include <cstdio>
@@ -131,8 +133,8 @@ int main(int argc, char** argv) {
     }
     printf("{\"n\": %d, \"passes\": %d, \"records\": %zu, \"depth\": %d, \"depth_seen\": %d, \"missing\": %lld, \"bad_union\": %lld, "
            "\"bad_leaf_box\": %lld, \"bad_dilated_union\": %lld, \"dilated_leaf_diff\": %lld, \"cost\": %.4f, \"host_sah_cost\": %.4f, "
-           "\"host_depth\": %d, \"ref_nodes\": %d}\n",
+           "\"host_depth\": %d, \"ref_depth\": %d, \"ref_nodes\": %d}\n",
            n, passes, rec.size(), max_depth, depth_seen, missing, bad_union, bad_leaf, bad_dil, dil_leaf_diff, cost, host_cost,
-           fb.max_depth, s->n_nodes);
+           fb.max_depth, wrt_scene_bvh_depth(h), s->n_nodes);
     return 0;
 }

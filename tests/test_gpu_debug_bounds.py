@@ -1,8 +1,9 @@
 """The bounds-checking build of the render core (libwrt_cuda_debug.so, -DWRT_DEBUG_BOUNDS): every ray-queue, request-queue,
 candidate-pool, node, coefficient and traversal-stack index is checked inside the kernels and a violation fails the
 frame with the source line.  compute-sanitizer is not available on the GPU pool, so this build is how the capacity
-arguments in kernels.cuh are checked: the 24 random scenes, the multi-batch / overflow / pool-full cases and the edge
-scenes all run under it, in a subprocess (the library is chosen at load time through WRT_CUDA_LIB)."""
+arguments in kernels.cuh are checked: the 24 random scenes, the multi-batch / overflow / pool-full cases, the edge
+scenes and the capacity-edge scenes (deep trees, stack budget, shadow crossings, list cap) all run under it, in a
+subprocess (the library is chosen at load time through WRT_CUDA_LIB)."""
 import os
 import subprocess
 import sys
@@ -20,10 +21,12 @@ def test_fuzz_and_overflow_cases_under_the_bounds_checking_build():
     env = dict(os.environ, WRT_CUDA_LIB=str(lib))
     sel = ("test_random_scene or test_multi_batch_frames_with_overflow or test_queue_overflow_is_rerendered or "
            "test_edge_scenes or test_soft_shadow_list_path_corner_cases or test_device_frame_overflow or "
-           "test_image_matches_oracle_and_reference")
+           "test_image_matches_oracle_and_reference or test_deep_tree or test_fan_walked_at_the_stack_budget or "
+           "test_hard_shadow_crossings or test_directional_crossings or test_soft_shadow_shafts_past_the_list_cap")
     p = subprocess.run([sys.executable, "-m", "pytest", str(REPO / "tests" / "test_gpu_fuzz.py"),
-                        str(REPO / "tests" / "test_gpu_parity.py"), "-m", "gpu", "-x", "-q", "-k", sel,
-                        "-p", "no:cacheprovider"], cwd=REPO, env=env, capture_output=True, text=True, timeout=1500)
+                        str(REPO / "tests" / "test_gpu_parity.py"), str(REPO / "tests" / "test_gpu_capacity_edges.py"),
+                        "-m", "gpu", "-x", "-q", "-k", sel, "-p", "no:cacheprovider"],
+                       cwd=REPO, env=env, capture_output=True, text=True, timeout=2700)
     assert p.returncode == 0, p.stdout[-4000:] + p.stderr[-2000:]
     assert " passed" in p.stdout and "WRT_DEBUG_BOUNDS" not in p.stdout
 

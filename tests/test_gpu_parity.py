@@ -336,6 +336,21 @@ sphere 4 1 -5 1.5
     r.ctx.close()
 
 
+_BANK_LIGHTS = ["light 3 6 4 1 0.3 0.3 0.3", "light 0.3 -1 -0.4 0 0.3 0.3 0.25", "attlight 1 7 7 1 0.4 0.4 0.4 0.5 0.02 0.001",
+                "light -4 5 3 1 0.3 0.2 0.2", "light -0.5 -1 0.3 0 0.2 0.3 0.2"]
+
+
+def light_bank(n, soft):
+    """The first n of a mix of point, attenuated and directional lights over two spheres (one glass) and a floor: the
+    kernels keep WRT_INLINE_LIGHTS = 4 lights in their parameters and read the rest from global memory."""
+    return ("imsize 96 64\neye 0 1 6\nviewdir 0 -0.1 -1\nhfov 60\nupdir 0 1 0\nbkgcolor 0.1 0.1 0.2 1.0\n"
+            + ("shadow soft\n" if soft else "") + "\n".join(_BANK_LIGHTS[:n]) + "\n"
+            + "mtlcolor 0.8 0.3 0.2 1 1 1 0.2 0.6 0.3 24 1 1.5\nsphere -1.5 0 -1 1.2\n"
+            + "mtlcolor 0.9 0.9 1.0 1 1 1 0.05 0.2 0.4 60 0.2 1.4\nsphere 1.4 0.2 0.5 1.0\n"
+            + "mtlcolor 0.4 0.7 0.4 1 1 1 0.2 0.7 0.1 10 1 1.0\n"
+            + "v -10 -1.2 8\nv 10 -1.2 8\nv 10 -1.2 -12\nv -10 -1.2 -12\nf 1 2 3\nf 1 3 4\n")
+
+
 @pytest.mark.parametrize("text,expect", [
     ("imsize 7 5\neye 0 0 0\nviewdir 0 0 -1\nupdir 0 1 0\nhfov 60\nbkgcolor 0.5 0.25 1 1\n", "empty"),
     ("imsize 33 17\neye 0 0 0\nviewdir 0 0 -1\nupdir 0 1 0\nhfov 60\nbkgcolor 0.1 0.1 0.1 1\nlight 1 1 1 1 1 1 1\n"
@@ -345,6 +360,8 @@ sphere 4 1 -5 1.5
     ("imsize 40 30\neye 0 0 0\nviewdir 0 0 -1\nupdir 0 1 0\nhfov 60\nbkgcolor 0.1 0.1 0.1 1\nlight 0 5 -3 1 1 1 1\nshadow soft\n"
      "mtlcolor 1 1 1 1 1 1 1 1 1 0 1 1\nsphere 0 5 -3 0.5\nmtlcolor 0.8 0.4 0.2 1 1 1 0.3 0.6 0.2 10 1 1\n"
      "sphere 0 0 -4 1\nv -5 -1 0\nv 5 -1 0\nv 0 -1 -9\nf 1 2 3\n", "light avatar + soft shadows (literal hasIntersection path)"),
+    (light_bank(4, soft=False), "4 lights, point and directional: the whole kernel-parameter light bank"),
+    (light_bank(5, soft=False), "5 lights: the 5th (directional) read from global memory"),
 ])
 def test_edge_scenes(workdir, text, expect):
     scene = Scene(text=text, asset_dir=workdir)
@@ -736,7 +753,8 @@ sphere -1.2 0.4 -0.5 0.4
 """
 
 
-@pytest.mark.parametrize("name,text", [("many_lights", MANY_LIGHTS), ("axis_aligned", AXIS_ALIGNED)])
+@pytest.mark.parametrize("name,text", [("many_lights", MANY_LIGHTS), ("axis_aligned", AXIS_ALIGNED),
+                                       ("bank_4", light_bank(4, soft=True)), ("bank_5", light_bank(5, soft=True))])
 def test_soft_shadow_list_path_corner_cases(workdir, monkeypatch, name, text):
     """Soft shadows through the candidate-list kernels, bit-compared with the oracle (which traces all 50 samples of
     every request): six area lights (more than the kernel-parameter light bank holds, attenuation included); an odd

@@ -878,7 +878,37 @@ int wrt_upload_scene(WrtContext* c, const WrtSceneDesc* s) {
 
     // ---- 3. trees ----
     int fast_depth = 0;
-    const bool host_build = c->host_bvh;
+    bool host_build = c->host_bvh;
+    // the host's binned-SAH build of fast_bvh.hpp into fnodes / dnodes / prim_box (synchronous)
+    auto build_on_host = [&]() -> int {
+        wrt::FastBvhBuilder& fbvh = c->fbvh;
+        fbvh.build(s);
+        if (fbvh.nodes.size() != (size_t)nn) return fail("wrt_upload_scene: fast BVH build failed");
+        std::vector<WrtNode> dil = fbvh.dilated(1e-3f, 1e-4f);
+        std::vector<float4> hb(2 * (size_t)np, make_float4(0.f, 0.f, 0.f, 0.f));
+        for (int i = 0; i < nn; i++) {
+            const WrtNode& nd = s->nodes[i];
+            if (nd.link >= 0 || i == 1) continue;
+            int p = ~nd.link;
+            if (p < 0 || p >= np) return fail("wrt_upload_scene: leaf link out of range");
+            hb[2 * (size_t)p] = make_float4(nd.pmin[0], nd.pmin[1], nd.pmin[2], 0.f);
+            hb[2 * (size_t)p + 1] = make_float4(nd.pmax[0], nd.pmax[1], nd.pmax[2], 0.f);
+        }
+        CK(cudaMemcpyAsync(fnodes, fbvh.nodes.data(), (size_t)nn * 32, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(dnodes, dil.data(), (size_t)nn * 32, cudaMemcpyHostToDevice, st));
+        CK(cudaMemcpyAsync(pbox, hb.data(), hb.size() * 16, cudaMemcpyHostToDevice, st));
+        CK(cudaStreamSynchronize(st));                  // the host vectors above go out of scope
+        fast_depth = fbvh.max_depth;
+        return 0;
+    };
+    // the per-octant and 4-wide copies of the walked tree, and the octant copies of the reference's tree
+    auto copy_walked_tree = [&](bool with_reference) {
+        const int g = (int)std::min<long long>(wide, (8ll * nn + 255) / 256);
+        c->launches += with_reference ? 3 : 2;
+        wrt::k_octant_copies<<<g, 256, 0, st>>>(fnodes, nn, onodes);
+        if (with_reference) wrt::k_octant_copies<<<g, 256, 0, st>>>(ds.nodes, nn, ronodes);
+        wrt::k_wide4_copies<<<(int)std::min<long long>(wide, (4ll * nn + 255) / 256), 256, 0, st>>>(onodes, nn, wnodes);
+    };
     auto t_b0 = std::chrono::steady_clock::now();
     if (np > 0 && !host_build) {
         wrt::BuildBuffers bb{};
@@ -910,34 +940,10 @@ int wrt_upload_scene(WrtContext* c, const WrtSceneDesc* s) {
         }
         wrt::k_bvh_layout<<<std::min(wide, (int)((n2 + 255) / 256)), 256, 0, st>>>(bb, np, fnodes, dnodes);
     } else if (np > 0) {
-        // WRT_HOST_BVH=1 (development A/B): the host's binned-SAH build of fast_bvh.hpp
-        wrt::FastBvhBuilder& fbvh = c->fbvh;
-        fbvh.build(s);
-        if (fbvh.nodes.size() != (size_t)nn) return fail("wrt_upload_scene: fast BVH build failed");
-        std::vector<WrtNode> dil = fbvh.dilated(1e-3f, 1e-4f);
-        std::vector<float4> hb(2 * (size_t)np, make_float4(0.f, 0.f, 0.f, 0.f));
-        for (int i = 0; i < nn; i++) {
-            const WrtNode& nd = s->nodes[i];
-            if (nd.link >= 0 || i == 1) continue;
-            int p = ~nd.link;
-            if (p < 0 || p >= np) return fail("wrt_upload_scene: leaf link out of range");
-            hb[2 * (size_t)p] = make_float4(nd.pmin[0], nd.pmin[1], nd.pmin[2], 0.f);
-            hb[2 * (size_t)p + 1] = make_float4(nd.pmax[0], nd.pmax[1], nd.pmax[2], 0.f);
-        }
-        CK(cudaMemcpyAsync(fnodes, fbvh.nodes.data(), (size_t)nn * 32, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(dnodes, dil.data(), (size_t)nn * 32, cudaMemcpyHostToDevice, st));
-        CK(cudaMemcpyAsync(pbox, hb.data(), hb.size() * 16, cudaMemcpyHostToDevice, st));
-        CK(cudaStreamSynchronize(st));                  // the host vectors above go out of scope
-        fast_depth = fbvh.max_depth;
+        // WRT_HOST_BVH=1 (development A/B)
+        if (build_on_host()) return 1;
     }
-    if (nn > 0) {
-        c->launches += 2;
-        const int g = (int)std::min<long long>(wide, (8ll * nn + 255) / 256);
-        wrt::k_octant_copies<<<g, 256, 0, st>>>(fnodes, nn, onodes);
-        wrt::k_octant_copies<<<g, 256, 0, st>>>(ds.nodes, nn, ronodes);
-        ++c->launches;
-        wrt::k_wide4_copies<<<(int)std::min<long long>(wide, (4ll * nn + 255) / 256), 256, 0, st>>>(onodes, nn, wnodes);
-    }
+    if (nn > 0) copy_walked_tree(true);
     CK(cudaGetLastError());
     unsigned* h_rb = c->h_counters + wrt::C_TOTAL;     // (the first C_TOTAL words belong to a frame that may still be in flight)
     CK(cudaMemcpyAsync(h_rb, d_flags, (wrt::BS_TOTAL + 8) * sizeof(int), cudaMemcpyDeviceToHost, st));
@@ -971,20 +977,40 @@ int wrt_upload_scene(WrtContext* c, const WrtSceneDesc* s) {
     // the strategy queries never read texels; a frame render needs every referenced map present
     c->textures_complete = !(flags & 2);
     // binary walks push at most one entry per level; the 4-wide walks (wide_bvh.h) descend two levels per node and push up
-    // to three
-    c->stack_rows = std::max(std::max(c->bvh_depth, fast_depth), 3 * ((fast_depth + 1) / 2)) + 2;
+    // to three.  90 rows x 128 threads x 4 B = 45 KB of dynamic shared memory per CTA: the reference's tree may be 88
+    // levels deep, the walked tree 58.
+    const int max_rows = 90;
+    auto rows_for = [&](int walked) { return std::max(std::max(c->bvh_depth, walked), 3 * ((walked + 1) / 2)) + 2; };
+    const int ploc_depth = host_build ? -1 : fast_depth;
+    if (np > 0 && !host_build && rows_for(fast_depth) > max_rows) {
+        // PLOC builds very deep trees over fans of triangles sharing a vertex and over boxes of very mixed sizes; the
+        // host's binned SAH stays shallow on them.  Results do not depend on the walked tree's shape (DESIGN.md section 4).
+        host_build = true;
+        if (build_on_host()) return 1;
+        copy_walked_tree(false);
+        CK(cudaGetLastError());
+        CK(cudaStreamSynchronize(st));
+        t_b1 = std::chrono::steady_clock::now();
+    }
+    c->stack_rows = rows_for(fast_depth);
 #ifdef WRT_DEBUG_BOUNDS
     if (const char* e = getenv("WRT_DEBUG_STACK_ROWS")) c->stack_rows = std::max(1, atoi(e));   // provoke the stack check (tests)
 #endif
-    if (c->stack_rows > 90)     // 90 rows x 128 threads x 4 B = 45 KB of dynamic shared memory per CTA
-        return fail("wrt_upload_scene: acceleration tree deeper than 88 levels (degenerate geometry?)");
+    if (c->stack_rows > max_rows)
+        return fail("wrt_upload_scene: acceleration tree too deep for the 90-row traversal stack (reference tree depth " +
+                    std::to_string(c->bvh_depth) + ", at most 88; walked tree depth " + std::to_string(fast_depth) +
+                    ", at most 58)");
     c->fast_depth = fast_depth;
     c->build_passes = state[wrt::BS_PASSES];
     c->has_scene = true;
-    if (getenv("WRT_VERBOSE"))
-        fprintf(stderr, "[wrt] upload: %d prims, %zu bytes staged, reference tree depth %d, walked tree depth %d (%s, %d PLOC passes), %.3f ms\n",
-                np, total, c->bvh_depth, fast_depth, host_build ? "host SAH" : "device PLOC", c->build_passes,
-                std::chrono::duration<double, std::milli>(t_b1 - t_b0).count());
+    if (getenv("WRT_VERBOSE")) {
+        char builder[96];
+        if (!host_build) snprintf(builder, sizeof builder, "device PLOC, %d passes", c->build_passes);
+        else if (c->host_bvh) snprintf(builder, sizeof builder, "host SAH");
+        else snprintf(builder, sizeof builder, "host SAH: the %d-pass PLOC tree was %d levels deep", c->build_passes, ploc_depth);
+        fprintf(stderr, "[wrt] upload: %d prims, %zu bytes staged, reference tree depth %d, walked tree depth %d (%s), %d stack rows, %.3f ms\n",
+                np, total, c->bvh_depth, fast_depth, builder, c->stack_rows, std::chrono::duration<double, std::milli>(t_b1 - t_b0).count());
+    }
     return 0;
 }
 

@@ -342,6 +342,68 @@ def f4_spheres_config(w: int = 3840, h: int = 2160, soft: bool = False) -> str:
     return "\n".join(lines) + "\n"
 
 
+# ---- geometry whose device-built (PLOC) tree is very deep: fans, slivers, nested sizes ----
+# Body lines only (v / f / sphere, no header, no mtlcolor); face indices start at vertex 1, so a body must come before
+# any other vertex of the config.  Numbers are fixed-point (%.6f): the config grammar rejects exponent notation.
+
+def _ring(n: int, y: float) -> list[str]:
+    return ["v %.6f %.6f %.6f" % (np.cos(2 * np.pi * i / n), y, np.sin(2 * np.pi * i / n)) for i in range(n)]
+
+
+def fan_geometry(n: int) -> str:
+    """A flat unit disc in y = 0 cut into n triangles that all share the centre vertex (0, 0, 0)."""
+    lines = ["v 0.000000 0.000000 0.000000"] + _ring(n, 0.0)
+    lines += ["f 1 %d %d" % (2 + i, 2 + (i + 1) % n) for i in range(n)]
+    return "\n".join(lines) + "\n"
+
+
+def cylinder_geometry(n: int) -> str:
+    """Radius 1, y from 0 to 2: n side quads (two triangles each) and a fan cap around each end's centre; 4n triangles."""
+    lines = ["v 0.000000 0.000000 0.000000", "v 0.000000 2.000000 0.000000"] + _ring(n, 0.0) + _ring(n, 2.0)
+    lo = lambda i: 3 + i % n                           # noqa: E731
+    hi = lambda i: 3 + n + i % n                       # noqa: E731
+    for i in range(n):
+        lines += ["f 1 %d %d" % (lo(i), lo(i + 1)), "f 2 %d %d" % (hi(i + 1), hi(i)),
+                  "f %d %d %d" % (lo(i), hi(i), hi(i + 1)), "f %d %d %d" % (lo(i), hi(i + 1), lo(i + 1))]
+    return "\n".join(lines) + "\n"
+
+
+def sliver_geometry(n: int = 4000) -> str:
+    """n thin triangles in z = 0 sharing the vertex (0, 0, 0), each 0.001 rad wide, spread around the full circle."""
+    lines = ["v 0.000000 0.000000 0.000000"]
+    for i in range(n):
+        a = 2 * np.pi * i / n
+        lines += ["v %.6f %.6f 0.000000" % (np.cos(a), np.sin(a)), "v %.6f %.6f 0.000000" % (np.cos(a + 0.001), np.sin(a + 0.001))]
+    lines += ["f 1 %d %d" % (2 + 2 * i, 3 + 2 * i) for i in range(n)]
+    return "\n".join(lines) + "\n"
+
+
+def mixed_radius_spheres(n: int = 5000, seed: int = 1) -> str:
+    """n spheres centred on the x axis in [-1, 1] with radii 10^U(-3, 2): tiny spheres nested inside huge ones."""
+    import random
+    rnd = random.Random(seed)
+    lines = []
+    for _ in range(n):
+        x = rnd.uniform(-1, 1)
+        lines.append("sphere %.6f 0 0 %.6f" % (x, 10 ** rnd.uniform(-3, 2)))
+    return "\n".join(lines) + "\n"
+
+
+def sphere_chain(n: int = 30) -> str:
+    """Sphere k at (1.5^k, 0, 0) with radius 0.4 * 1.5^k: every sphere is larger than all the ones before it together."""
+    return "".join("sphere %.6f 0 0 %.6f\n" % (1.5 ** k, 0.4 * 1.5 ** k) for k in range(n))
+
+
+DEEP_TREE_GEOMETRY = {
+    "fan_1000": lambda: fan_geometry(1000),
+    "fan_2000": lambda: fan_geometry(2000),
+    "cylinder_2000": lambda: cylinder_geometry(2000),
+    "slivers_4000": lambda: sliver_geometry(4000),
+    "mixed_radii_5000": lambda: mixed_radius_spheres(5000, 1),
+    "chain_30": lambda: sphere_chain(30),
+}
+
+
 # BASELINE.json `configs`, in order.  (name, config text builder kwargs, uses bunny, soft)
 BENCH_CONFIGS = {
     "config": dict(builder=bunny_shadow_config, w=800, h=600, soft=False),
