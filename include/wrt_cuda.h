@@ -88,10 +88,22 @@ int wrt_trace_closest(WrtContext* ctx, const float* orig, const float* dir, int6
  * so that the parity tests can hold the frame kernel itself to the oracle on arbitrary ray batches
  * (IIntersectStrategy::UpdateInter, include/IIntersectStrategy.h:10-11). */
 int wrt_trace_closest_wavefront(WrtContext* ctx, const float* orig, const float* dir, int64_t n, WrtHit* hits);
+/* Shadow requests answered by the kernels a frame answers its own with (k_shadow_hard; k_soft_lists -> k_soft_filter ->
+ * k_soft_list_rays, or k_shadow_soft; k_shadow_directional), for the parity tests.  Request i is the shading point pos[i]
+ * with normal ndir[i] and scene light light[i]; pixel[i] and path[i] (a ray-tree path id >= 1) key the soft-shadow RNG,
+ * self_object[i] is the object a directional-light request's point lies on.  The requests are queued in input order into
+ * request queue `queue` (0: level 0, 1: levels 1..5, 2: deeper) exactly as the frame's surface stage queues them and run on
+ * that queue's stream and grid.  With WRT_REQ_SHAFT_CULL, soft requests whose shaft to the light is empty are answered by
+ * the surface stage's shaft test instead, as on level 0.  coeff[i] is what the frame stores: the hard-shadow or
+ * directional product, or the number of lit samples of 50 (as a float).  Kernel timing, when on, covers these launches. */
+#define WRT_REQ_SHAFT_CULL 1
+int wrt_shadow_requests_wavefront(WrtContext* ctx, int queue, int flags, const float* pos, const float* ndir, const int32_t* light,
+                                  const uint32_t* pixel, const uint32_t* path, const int32_t* self_object, int64_t n, float* coeff);
 /* BVHStrategy::getShadowCoeffi / ShadowHelper (include/BVHStrategy.hpp:13-48): the product of (1 - alpha) over the blocking
  * leaves, multiplied in the association of the caller's tree (`l * r` at every inner node) — the reference's float bit
  * for bit, whichever tree the kernel walks (csrc/cuda/shadow_assoc.h; beyond 12 translucent crossings on one ray or a
- * tree deeper than 64 levels: the same factors in visit order). */
+ * tree deeper than 64 levels: the same factors in visit order).  The frame's kernel is held to the same bar, request by
+ * request, through wrt_shadow_requests_wavefront (tests/test_gpu_shadow_requests.py). */
 int wrt_shadow_hard(WrtContext* ctx, const float* pos, const float* ndir, const float* lightpos, int64_t n, float* coeff);
 int wrt_shadow_soft(WrtContext* ctx, const float* pos, const float* ndir, const float* lightpos, int64_t n, float* coeff);
 int wrt_shadow_directional(WrtContext* ctx, const float* pos, const int32_t* self_object, const float* lightdir4,

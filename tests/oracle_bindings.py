@@ -41,6 +41,7 @@ def oracle():
         lib.orc_render_rect.argtypes = [dp, C.POINTER(cabi.WrtCamera), u32, i32, i32, i32, i32, i32, i32, i32, vp, vp,
                                         C.POINTER(cabi.WrtStats)]
         lib.orc_light_sample_uv.argtypes = [u32, u32, u32, u32, u32, vp]
+        lib.orc_shadow_requests.argtypes = [dp, u32, vp, vp, vp, vp, vp, vp, i64, vp]
         _orc = lib
     return _orc
 
@@ -80,6 +81,20 @@ class OracleScene:
         out = np.zeros(len(pos), dtype=np.float32)
         self.lib.orc_shadow_directional(self.scene.desc_ptr, pos.ctypes.data, so.ctypes.data, lightdir4.ctypes.data,
                                         len(pos), out.ctypes.data)
+        return out
+
+    def shadow_requests(self, pos, ndir, light, pixel, path, self_object, seed=cabi.WRT_DEFAULT_SEED):
+        """What a frame stores for each shadow request (point, normal, scene light): the hard-shadow coefficient, the number
+        of lit soft-shadow samples of 50 (RNG keyed on pixel and path) or the directional product."""
+        pos, ndir = _f32(pos), _f32(ndir)
+        li = np.ascontiguousarray(light, dtype=np.int32)
+        px, pa = np.ascontiguousarray(pixel, dtype=np.uint32), np.ascontiguousarray(path, dtype=np.uint32)
+        so = np.ascontiguousarray(self_object, dtype=np.int32)
+        assert len(pos) == len(ndir) == len(li) == len(px) == len(pa) == len(so)
+        assert ((li >= 0) & (li < self.scene.desc.n_lights)).all()
+        out = np.zeros(len(pos), dtype=np.float32)
+        self.lib.orc_shadow_requests(self.scene.desc_ptr, seed, pos.ctypes.data, ndir.ctypes.data, li.ctypes.data,
+                                     px.ctypes.data, pa.ctypes.data, so.ctypes.data, len(pos), out.ctypes.data)
         return out
 
     def trace_ray(self, orig, dirs, depth=None, pixel=None, seed=cabi.WRT_DEFAULT_SEED):

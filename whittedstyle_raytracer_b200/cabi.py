@@ -17,6 +17,7 @@ CUDA_LIB = PKG / "libwrt_cuda.so"
 WRT_MAX_DEPTH = 9
 WRT_SOFT_SAMPLES = 50
 WRT_DEFAULT_SEED = 0x5EED
+WRT_REQ_SHAFT_CULL = 1          # wrt_shadow_requests_wavefront: answer soft requests with an empty shaft by the shaft test
 
 
 class WrtNode(C.Structure):
@@ -88,7 +89,8 @@ HOST_SYMBOLS = [
 # Entry points include/wrt_cuda.h declares
 CUDA_SYMBOLS = [
     "wrt_create", "wrt_destroy", "wrt_last_error", "wrt_upload_scene", "wrt_set_camera", "wrt_set_tiles",
-    "wrt_set_options", "wrt_enable_kernel_timing", "wrt_trace_closest", "wrt_trace_closest_wavefront", "wrt_shadow_hard", "wrt_shadow_soft", "wrt_shadow_directional",
+    "wrt_set_options", "wrt_enable_kernel_timing", "wrt_trace_closest", "wrt_trace_closest_wavefront", "wrt_shadow_requests_wavefront",
+    "wrt_shadow_hard", "wrt_shadow_soft", "wrt_shadow_directional",
     "wrt_render", "wrt_render_device", "wrt_finish_device", "wrt_get_stats", "wrt_tile_pixel_count",
     "wrt_scatter_tiles", "wrt_kernel_launch_count", "wrt_get_kernel_times", "wrt_get_kernel_launches", "wrt_measure_fp32_peak",
     "wrt_multi_create", "wrt_multi_destroy", "wrt_multi_device_count", "wrt_multi_context", "wrt_multi_uses_peer_stores",
@@ -153,6 +155,7 @@ def load_cuda() -> C.CDLL:
         lib.wrt_set_options.argtypes = [vp, i32, u32, C.c_float]
         lib.wrt_trace_closest.argtypes = [vp, vp, vp, i64, vp]
         lib.wrt_trace_closest_wavefront.argtypes = [vp, vp, vp, i64, vp]
+        lib.wrt_shadow_requests_wavefront.argtypes = [vp, i32, i32, vp, vp, vp, vp, vp, vp, i64, vp]
         lib.wrt_shadow_hard.argtypes = [vp, vp, vp, vp, i64, vp]
         lib.wrt_shadow_soft.argtypes = [vp, vp, vp, vp, i64, vp]
         lib.wrt_shadow_directional.argtypes = [vp, vp, vp, vp, i64, vp]

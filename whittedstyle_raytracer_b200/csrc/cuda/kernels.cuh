@@ -1438,6 +1438,78 @@ __global__ void __launch_bounds__(256) k_unpack_hits(const __grid_constant__ Dev
     }
 }
 
+// ---- shadow requests answered by the FRAME's shadow kernels (wrt_shadow_requests_wavefront: the tests put their
+// requests through k_shadow_hard, the candidate-list kernels, k_shadow_soft and k_shadow_directional themselves) ----
+struct ShadowRequestIn {
+    float pos[3], ndir[3];
+    int light;                 // scene light index
+    unsigned pixel, path;      // soft-shadow RNG key (point lights)
+    int self_object;           // directional lights: the object the point lies on
+    int slot;                  // position in its request queue (host-assigned, input order); -1: answered by the shaft test
+    int pad;
+};
+
+// kind[i]: 0 directional light, 1 point light, 2 soft point-light request answered by the spawn-time shaft test of
+// surface_warp (WRT_CULL_SHAFT, only with shaft_cull != 0): its whole shaft to the area light misses every leaf box.
+__global__ void __launch_bounds__(128) k_classify_shadow_requests(const __grid_constant__ DevScene s, const ShadowRequestIn* in,
+                                                                 long long n, int shaft_cull, unsigned char* kind) {
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+        const ShadowRequestIn r = in[i];
+        const WrtLight* L = s.lights + r.light;
+        unsigned char k = 0;
+        if (float_equal(L->pos[3], 1.f)) {
+            k = 1;
+            if (shaft_cull && s.shadow_type != 0) {
+                const f3 sorig = mk3(r.pos[0], r.pos[1], r.pos[2]) + 0.0005f * mk3(r.ndir[0], r.ndir[1], r.ndir[2]);
+                const float so[3] = {sorig.x, sorig.y, sorig.z};
+                float tri[9];
+                for (int j = 0; j < 9; j++) tri[j] = L->tri[j];
+                if (wrt_shaft_is_empty(s.onodes, s.n_nodes, so, tri)) k = 2;
+            }
+        }
+        kind[i] = k;
+    }
+}
+
+// Queues requests [0, n) of `in` into request queue q exactly as surface_warp writes them: node id = index, shadow-ray
+// origin pos + 0.0005 * nDir, coefficient slot 0 (50 for a request the shaft test answered); then sets the queue lengths.
+__global__ void __launch_bounds__(256) k_pack_shadow_requests(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
+                                                              int q, const ShadowRequestIn* in, unsigned n, unsigned n_point,
+                                                              unsigned n_dir) {
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        const ShadowRequestIn r = in[i];
+        const unsigned li = (unsigned)r.light;
+        const f3 pos = mk3(r.pos[0], r.pos[1], r.pos[2]), nDir = mk3(r.ndir[0], r.ndir[1], r.ndir[2]);
+        const f3 sorig = pos + 0.0005f * nDir;                         // BVHStrategy.hpp:15, Renderer.hpp:349
+        if (WRT_IN_BOUNDS((size_t)i * s.n_lights + li, (size_t)fb.n_node_cap * s.n_lights))
+            fb.coeff[(size_t)i * s.n_lights + li] = r.slot < 0 ? (float)WRT_SOFT_SAMPLES : 0.f;
+        if (r.slot < 0) continue;
+        const unsigned slot = (unsigned)r.slot;
+        if (float_equal(s.lights[li].pos[3], 1.f)) {
+            if (WRT_IN_BOUNDS(slot, fb.preq_cap[q])) {
+                fb.preq_o[q][slot] = make_float4(sorig.x, sorig.y, sorig.z, __uint_as_float(i));
+                fb.preq_k[q][slot] = make_uint4(li, r.pixel, r.path, 0u);
+            }
+        } else {
+            const int prim = (r.self_object >= 0 && r.self_object < s.n_prims) ? __ldg(s.object_prim + r.self_object) : -1;
+            if (WRT_IN_BOUNDS(slot, fb.dreq_cap[q])) {
+                fb.dreq_o[q][slot] = make_float4(pos.x, pos.y, pos.z, __uint_as_float(i));
+                fb.dreq_k[q][slot] = make_uint4(li, (unsigned)prim, 0u, 0u);
+            }
+        }
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) {
+        fb.counters[C_NPREQ + q] = n_point;
+        fb.counters[C_NDREQ + q] = n_dir;
+    }
+}
+
+__global__ void __launch_bounds__(256) k_unpack_shadow_requests(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
+                                                                const ShadowRequestIn* in, unsigned n, float* out) {
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        out[i] = fb.coeff[(size_t)i * s.n_lights + (unsigned)in[i].light];
+}
+
 // mode 0: BVHStrategy::getShadowCoeffi (hard); mode 1: Renderer::getShadowCoeffi(Vector3f&) (soft sample)
 __global__ void __launch_bounds__(128) k_batch_shadow(DevScene s, const float* pos, const float* ndir, const float* lightpos,
                                                       long long n, float* out, int mode, float prune_rel) {

@@ -610,6 +610,8 @@ int render_all(WrtContext* c, cudaStream_t user, bool join_user, uint8_t* d_imag
     return 0;
 }
 
+void tally_kernel_times(WrtContext* c);
+
 int finish_frame(WrtContext* c) {
     cudaStream_t st = c->chain;
     CK(cudaStreamSynchronize(st));
@@ -639,6 +641,12 @@ int finish_frame(WrtContext* c) {
     if (check_debug_bounds()) return 1;
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, c->ev_begin, c->ev_end) == cudaSuccess) c->stats.gpu_ms = ms;
+    tally_kernel_times(c);
+    return 0;
+}
+
+// Per-family times and launch counts of the timed launches since c->timed was cleared (ev_begin: their common start).
+void tally_kernel_times(WrtContext* c) {
     for (float& f : c->family_ms) f = 0.f;
     for (int& n : c->family_launches) n = 0;
     const bool dump = getenv("WRT_TIMING_DUMP") != nullptr;      // development: every timed launch, in enqueue order
@@ -653,7 +661,6 @@ int finish_frame(WrtContext* c) {
                     tl.on_chain ? "chain" : "side", t0 * 1e3f, t1 * 1e3f);
         }
     }
-    return 0;
 }
 
 } // namespace
@@ -1164,6 +1171,77 @@ int wrt_shadow_directional(WrtContext* c, const float* pos, const int32_t* self_
     CK(cudaMemcpyAsync(coeff, c->d_scratch[3], (size_t)n * 4, cudaMemcpyDeviceToHost, st));
     CK(cudaStreamSynchronize(st));
     return 0;
+}
+
+// Shadow requests answered by the frame's own shadow kernels: queued into request queue `queue` in input order, exactly as
+// k_surface_spawn queues them (one ray-tree node per request), and run by enqueue_shadows on the stream and grid a frame
+// uses for that queue.  The result is what the frame stores for the (node, light) pair.
+int wrt_shadow_requests_wavefront(WrtContext* c, int queue, int flags, const float* pos, const float* ndir, const int32_t* light,
+                                  const uint32_t* pixel, const uint32_t* path, const int32_t* self_object, int64_t n, float* coeff) {
+    if (batch_common(c, n)) return 1;
+    if (queue < 0 || queue >= WRT_QUEUES) return fail("wrt_shadow_requests_wavefront: queue out of range");
+    if (n == 0) return 0;
+    if (!pos || !ndir || !light || !pixel || !path || !self_object || !coeff) return fail("wrt_shadow_requests_wavefront: null argument");
+    std::vector<wrt::ShadowRequestIn> req((size_t)n);
+    for (int64_t i = 0; i < n; i++) {
+        if (light[i] < 0 || light[i] >= c->ds.n_lights) return fail("wrt_shadow_requests_wavefront: light index out of range");
+        wrt::ShadowRequestIn& r = req[i];
+        for (int k = 0; k < 3; k++) { r.pos[k] = pos[3 * i + k]; r.ndir[k] = ndir[3 * i + k]; }
+        r.light = light[i]; r.pixel = pixel[i]; r.path = path[i]; r.self_object = self_object[i];
+        r.slot = -1; r.pad = 0;
+    }
+    if (c->frame_pending && finish_frame(c)) return 1;
+    if (ensure_frame_buffers(c, std::max(c->batch_slots, 1u << 20))) return 1;
+    wrt::FrameBuffers& fb = c->fb;
+    // the frame's streams: queues 0 and 1 on the side stream (when the frame overlaps them), queue 2 on the chain
+    const bool overlap = c->overlap && (!c->kernel_timing || getenv("WRT_TIMING_OVERLAP") != nullptr);
+    cudaStream_t st = queue < 2 && overlap ? c->side : c->chain;
+    const size_t in_bytes = (size_t)n * sizeof(wrt::ShadowRequestIn);
+    if (ensure_scratch(c, 0, in_bytes) || ensure_scratch(c, 1, (size_t)n) || ensure_scratch(c, 2, (size_t)n * sizeof(float))) return 1;
+    wrt::ShadowRequestIn* d_in = (wrt::ShadowRequestIn*)c->d_scratch[0];
+    unsigned char* d_kind = (unsigned char*)c->d_scratch[1];
+    float* d_out = (float*)c->d_scratch[2];
+    if (c->kernel_timing) {
+        c->timed.clear();
+        c->event_next = 0;
+        CK(cudaEventRecord(c->ev_begin, st));
+    }
+    // point or directional light, and the spawn-time shaft test; the host then assigns the queue slots in input order
+    CK(cudaMemcpyAsync(d_in, req.data(), in_bytes, cudaMemcpyHostToDevice, st));
+    ++c->launches;
+    wrt::k_classify_shadow_requests<<<(int)std::min<int64_t>((n + 127) / 128, grid_for(c, 8)), 128, 0, st>>>(
+        c->ds, d_in, n, (flags & WRT_REQ_SHAFT_CULL) ? 1 : 0, d_kind);
+    CK(cudaGetLastError());
+    std::vector<unsigned char> kind((size_t)n);
+    CK(cudaMemcpyAsync(kind.data(), d_kind, (size_t)n, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    // one node per request: a chunk fits the queue, the nodes, and the list kernels' 32-bit ray index (nreq * 50 < 2^32)
+    const int64_t chunk = (int64_t)std::min<unsigned long long>(
+        {(unsigned long long)fb.preq_cap[queue], (unsigned long long)fb.dreq_cap[queue], (unsigned long long)fb.n_node_cap,
+         ((1ull << 32) - 1) / WRT_SOFT_SAMPLES});
+    std::vector<std::pair<unsigned, unsigned>> counts;
+    for (int64_t off = 0; off < n; off += chunk) {
+        unsigned np = 0, nd = 0;
+        for (int64_t i = off; i < std::min(n, off + chunk); i++)
+            req[i].slot = kind[i] == 0 ? (int)nd++ : (kind[i] == 1 ? (int)np++ : -1);
+        counts.push_back({np, nd});
+    }
+    CK(cudaMemcpyAsync(d_in, req.data(), in_bytes, cudaMemcpyHostToDevice, st));
+    for (int64_t off = 0, k = 0; off < n; off += chunk, k++) {
+        const unsigned m = (unsigned)std::min<int64_t>(chunk, n - off);
+        CK(cudaMemsetAsync(fb.counters, 0, wrt::C_TOTAL * sizeof(unsigned), st));
+        ++c->launches;
+        wrt::k_pack_shadow_requests<<<grid_for(c, 4), 256, 0, st>>>(c->ds, fb, queue, d_in + off, m, counts[k].first, counts[k].second);
+        int work_seq = 0;
+        if (enqueue_shadows(c, st, queue, work_seq)) return 1;
+        ++c->launches;
+        wrt::k_unpack_shadow_requests<<<grid_for(c, 4), 256, 0, st>>>(c->ds, fb, d_in + off, m, d_out + off);
+        CK(cudaGetLastError());
+    }
+    CK(cudaMemcpyAsync(coeff, d_out, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    if (c->kernel_timing) tally_kernel_times(c);
+    return check_debug_bounds();
 }
 
 // ---------------- frame ----------------

@@ -132,6 +132,23 @@ class CudaStrategy:
         self.ctx._check(self.ctx.lib.wrt_trace_closest_wavefront(self.ctx.h, o.ctypes.data, d.ctypes.data, len(o), out.ctypes.data))
         return out
 
+    def shadowRequestsWavefront(self, pos, nDir, light, pixel, path, self_object, queue=0, flags=0) -> np.ndarray:
+        """Test entry: shadow requests (point, normal, scene light index) answered by the frame's own shadow kernels of
+        request queue `queue` (wrt_shadow_requests_wavefront).  Per request what the frame stores: the hard-shadow
+        coefficient, the lit samples of 50 for soft shadows (RNG keyed on pixel and path), the directional product
+        (self_object: the point's object).  flags: cabi.WRT_REQ_SHAFT_CULL answers empty soft shafts by the shaft test."""
+        p, n = _f32(pos, 3), _f32(nDir, 3)
+        li = np.ascontiguousarray(light, dtype=np.int32)
+        px, pa = np.ascontiguousarray(pixel, dtype=np.uint32), np.ascontiguousarray(path, dtype=np.uint32)
+        so = np.ascontiguousarray(self_object, dtype=np.int32)
+        if not (len(p) == len(n) == len(li) == len(px) == len(pa) == len(so)):
+            raise ValueError("shadowRequestsWavefront: arrays of different lengths")
+        out = np.zeros(len(p), dtype=np.float32)
+        self.ctx._check(self.ctx.lib.wrt_shadow_requests_wavefront(
+            self.ctx.h, queue, flags, p.ctypes.data, n.ctypes.data, li.ctypes.data, px.ctypes.data, pa.ctypes.data,
+            so.ctypes.data, len(p), out.ctypes.data))
+        return out
+
     def getShadowCoeffi(self, pos, nDir, lightpos) -> np.ndarray:
         """Hard-shadow coefficient per (hit point, shading normal, light position)."""
         return self._shadow(self.ctx.lib.wrt_shadow_hard, pos, nDir, lightpos)
