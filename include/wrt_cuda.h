@@ -114,6 +114,13 @@ int wrt_shadow_directional(WrtContext* ctx, const float* pos, const int32_t* sel
  * pixels of other ranks' tiles left untouched) to host memory.  Synchronous. */
 int wrt_render(WrtContext* ctx, uint8_t* rgb_host, WrtStats* stats);
 
+/* The frame wrt_render renders, and also its unquantised colour: rgb_f_host (width*height*3 float, row-major) receives
+ * the level-0 colour k_combine_resolve quantises (Renderer.hpp:259, before `255 * min(c, 1)`); pixels of other ranks'
+ * tiles are left untouched in both buffers.  After each batch's combine one device-to-host copy of the batch's level-0
+ * nodes is queued on the frame's stream (a batch re-rendered after a queue overflow copies again, over its first
+ * attempt); wrt_render and wrt_render_device queue no such copy.  Synchronous. */
+int wrt_render_float(WrtContext* ctx, float* rgb_f_host, uint8_t* rgb_host, WrtStats* stats);
+
 /* Asynchronous form on caller-provided device memory and stream (cudaStream_t as void*;
  * NULL is CUDA's legacy default stream, e.g. torch's default current stream).  d_rgb_tiles receives this rank's pixels in tile
  * order: wrt_tile_pixel_count(ctx, rank, world) * 3 bytes.  Call wrt_finish_device()

@@ -13,10 +13,12 @@ from whittedstyle_raytracer_b200 import cabi
 
 REPO = Path(__file__).resolve().parent.parent
 ORACLE_LIB = REPO / "oracle" / "liboracle.so"
+# the same source built with -DORC_DEVICE_MATH: powf / acosf / atan2f as the render core evaluates them
+ORACLE_DEVMATH_LIB = REPO / "oracle" / "liboracle_devmath.so"
 REF_LIB = REPO / "oracle" / "_ref" / "libwhitted_ref.so"
 REF_EXE = REPO / "oracle" / "_ref" / "whitted_ref"
 
-_orc = None
+_orc = {}
 _ref = None
 
 
@@ -24,10 +26,9 @@ def _f32(a):
     return np.ascontiguousarray(a, dtype=np.float32)
 
 
-def oracle():
-    global _orc
-    if _orc is None:
-        lib = C.CDLL(str(ORACLE_LIB))
+def oracle(device_math=False):
+    if device_math not in _orc:
+        lib = C.CDLL(str(ORACLE_DEVMATH_LIB if device_math else ORACLE_LIB))
         vp, i64, u32, i32 = C.c_void_p, C.c_int64, C.c_uint32, C.c_int
         dp = C.POINTER(cabi.WrtSceneDesc)
         lib.orc_trace_closest.argtypes = [dp, vp, vp, i64, vp]
@@ -42,8 +43,8 @@ def oracle():
                                         C.POINTER(cabi.WrtStats)]
         lib.orc_light_sample_uv.argtypes = [u32, u32, u32, u32, u32, vp]
         lib.orc_shadow_requests.argtypes = [dp, u32, vp, vp, vp, vp, vp, vp, i64, vp]
-        _orc = lib
-    return _orc
+        _orc[device_math] = lib
+    return _orc[device_math]
 
 
 def have_reference() -> bool:
@@ -51,11 +52,12 @@ def have_reference() -> bool:
 
 
 class OracleScene:
-    """The oracle over a whittedstyle_raytracer_b200.Scene."""
+    """The oracle over a whittedstyle_raytracer_b200.Scene.  device_math=True: the liboracle_devmath.so build, whose
+    powf / acosf / atan2f are the render core's (everything else is the same source)."""
 
-    def __init__(self, scene):
+    def __init__(self, scene, device_math=False):
         self.scene = scene
-        self.lib = oracle()
+        self.lib = oracle(device_math)
 
     def trace_closest(self, orig, dirs):
         orig, dirs = _f32(orig), _f32(dirs)

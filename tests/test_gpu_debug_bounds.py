@@ -2,8 +2,9 @@
 candidate-pool, node, coefficient and traversal-stack index is checked inside the kernels and a violation fails the
 frame with the source line.  compute-sanitizer is not available on the GPU pool, so this build is how the capacity
 arguments in kernels.cuh are checked: the 24 random scenes, the multi-batch / overflow / pool-full cases, the edge
-scenes, the capacity-edge scenes (deep trees, stack budget, shadow crossings, list cap) and the frame's shadow kernels on
-given requests (tests/test_gpu_shadow_requests.py) all run under it, in a
+scenes, the capacity-edge scenes (deep trees, stack budget, shadow crossings, list cap), the frame's shadow kernels on
+given requests (tests/test_gpu_shadow_requests.py) and the float-frame shading edges, overflow and tile cases
+(tests/test_gpu_float_frame.py) all run under it, in a
 subprocess (the library is chosen at load time through WRT_CUDA_LIB)."""
 import os
 import subprocess
@@ -24,10 +25,11 @@ def test_fuzz_and_overflow_cases_under_the_bounds_checking_build():
            "test_edge_scenes or test_soft_shadow_list_path_corner_cases or test_device_frame_overflow or "
            "test_image_matches_oracle_and_reference or test_deep_tree or test_fan_walked_at_the_stack_budget or "
            "test_hard_shadow_crossings or test_directional_crossings or test_soft_shadow_shafts_past_the_list_cap or "
-           "test_shadow_requests")
+           "test_shadow_requests or test_float_frame_shading_edges or test_float_frame_overflow or test_float_frame_tiles or "
+           "test_float_frame_forty_lights")
     p = subprocess.run([sys.executable, "-m", "pytest", str(REPO / "tests" / "test_gpu_fuzz.py"),
                         str(REPO / "tests" / "test_gpu_parity.py"), str(REPO / "tests" / "test_gpu_capacity_edges.py"),
-                        str(REPO / "tests" / "test_gpu_shadow_requests.py"),
+                        str(REPO / "tests" / "test_gpu_shadow_requests.py"), str(REPO / "tests" / "test_gpu_float_frame.py"),
                         "-m", "gpu", "-x", "-q", "-k", sel, "-p", "no:cacheprovider"],
                        cwd=REPO, env=env, capture_output=True, text=True, timeout=2700)
     assert p.returncode == 0, p.stdout[-4000:] + p.stderr[-2000:]

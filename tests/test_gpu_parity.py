@@ -351,7 +351,7 @@ def light_bank(n, soft):
             + "v -10 -1.2 8\nv 10 -1.2 8\nv 10 -1.2 -12\nv -10 -1.2 -12\nf 1 2 3\nf 1 3 4\n")
 
 
-@pytest.mark.parametrize("text,expect", [
+EDGE_SCENES = [
     ("imsize 7 5\neye 0 0 0\nviewdir 0 0 -1\nupdir 0 1 0\nhfov 60\nbkgcolor 0.5 0.25 1 1\n", "empty"),
     ("imsize 33 17\neye 0 0 0\nviewdir 0 0 -1\nupdir 0 1 0\nhfov 60\nbkgcolor 0.1 0.1 0.1 1\nlight 1 1 1 1 1 1 1\n"
      "mtlcolor 0.8 0.4 0.2 1 1 1 0.3 0.6 0.2 10 1 1\nsphere 0 0 -3 1\n", "one object (root is a leaf)"),
@@ -362,7 +362,10 @@ def light_bank(n, soft):
      "sphere 0 0 -4 1\nv -5 -1 0\nv 5 -1 0\nv 0 -1 -9\nf 1 2 3\n", "light avatar + soft shadows (literal hasIntersection path)"),
     (light_bank(4, soft=False), "4 lights, point and directional: the whole kernel-parameter light bank"),
     (light_bank(5, soft=False), "5 lights: the 5th (directional) read from global memory"),
-])
+]
+
+
+@pytest.mark.parametrize("text,expect", EDGE_SCENES)
 def test_edge_scenes(workdir, text, expect):
     scene = Scene(text=text, asset_dir=workdir)
     ref, ost = ob.OracleScene(scene).render()

@@ -124,6 +124,9 @@ struct WrtContext {
     size_t d_image_bytes = 0;
     uint8_t* h_image = nullptr;        // pinned staging
     size_t h_image_bytes = 0;
+    float4* h_float = nullptr;         // pinned, slot order: level-0 {colour, fr} of every local slot (wrt_render_float)
+    size_t h_float_bytes = 0;
+    bool copy_float = false;           // set for the duration of wrt_render_float: each batch copies its level 0 to h_float
 
     // batch-query scratch
     void* d_scratch[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -473,6 +476,8 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
         void* args[] = {(void*)&ds, (void*)&fb, (void*)&tm, (void*)&slot0, (void*)&n, (void*)&shade_from, (void*)&d_image, (void*)&d_packed};
         CK(cudaLaunchCooperativeKernel((const void*)k_combine_resolve, dim3(c->coop_grid), dim3(256), args, 0, st));
     }
+    if (c->copy_float)                                 // the combined level-0 colours this batch quantised, in slot order
+        CK(cudaMemcpyAsync(c->h_float + slot0, fb.node_a, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, st));
     CK(cudaGetLastError());
     if (C_WORK + 2 * work_seq > C_TOTAL) return fail("internal: work counters exceed the counter block");
     return 0;
@@ -750,6 +755,7 @@ void wrt_destroy(WrtContext* c) {
     for (int k = 0; k < 5; k++) if (c->d_scratch[k]) cudaFree(c->d_scratch[k]);
     if (c->d_image) cudaFree(c->d_image);
     if (c->h_image) cudaFreeHost(c->h_image);
+    if (c->h_float) cudaFreeHost(c->h_float);
     if (c->h_counters) cudaFreeHost(c->h_counters);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     for (cudaEvent_t e : c->event_pool) cudaEventDestroy(e);
@@ -1294,6 +1300,33 @@ int wrt_render(WrtContext* c, uint8_t* rgb_host, WrtStats* stats) {
         }
     }
     if (stats) *stats = c->stats;
+    return 0;
+}
+
+int wrt_render_float(WrtContext* c, float* rgb_f_host, uint8_t* rgb_host, WrtStats* stats) {
+    if (!c || !rgb_f_host || !rgb_host) return fail("wrt_render_float: null argument");
+    CK(cudaSetDevice(c->device));
+    if (!c->has_cam) return fail("wrt_render_float: no camera set");
+    const long long slots = c->local_slots(c->rank, c->world);
+    const size_t bytes = (size_t)std::max(slots, 1ll) * sizeof(float4);
+    if (c->h_float_bytes < bytes) {
+        if (c->h_float) cudaFreeHost(c->h_float);
+        c->h_float = nullptr; c->h_float_bytes = 0;
+        CK(cudaMallocHost((void**)&c->h_float, bytes));
+        c->h_float_bytes = bytes;
+    }
+    c->copy_float = true;
+    const int rc = wrt_render(c, rgb_host, stats);     // synchronous: every batch's copy has landed when it returns
+    c->copy_float = false;
+    if (rc) return rc;
+    wrt::TileMap tm = c->tilemap();
+    for (long long s = 0; s < slots; s++) {
+        int x, y;
+        if (tm.slot_to_pixel(s, c->rank, x, y)) {
+            float* p = rgb_f_host + 3 * ((size_t)y * tm.width + x);
+            p[0] = c->h_float[s].x; p[1] = c->h_float[s].y; p[2] = c->h_float[s].z;
+        }
+    }
     return 0;
 }
 

@@ -191,6 +191,22 @@ class Renderer:
         self.last_stats = stats_dict(st)
         return out
 
+    def render_float(self, out_f: np.ndarray | None = None, out: np.ndarray | None = None) -> tuple[np.ndarray, np.ndarray]:
+        """The frame render() renders, with its unquantised colour: ((H, W, 3) float32, (H, W, 3) uint8).  The float image
+        is what the 8-bit one quantises as int(255 * min(c, 1)), clamped to [0, 255]; with tiles only this rank's pixels
+        are written."""
+        cam = self.scene.camera
+        if out_f is None:
+            out_f = np.zeros((cam.height, cam.width, 3), np.float32)
+        if out is None:
+            out = np.zeros((cam.height, cam.width, 3), np.uint8)
+        if out_f.dtype != np.float32 or out_f.shape != (cam.height, cam.width, 3) or not out_f.flags.c_contiguous:
+            raise ValueError("render_float: out_f must be a C-contiguous (H, W, 3) float32 array")
+        st = cabi.WrtStats()
+        self.ctx._check(self.ctx.lib.wrt_render_float(self.ctx.h, out_f.ctypes.data, out.ctypes.data, C.byref(st)))
+        self.last_stats = stats_dict(st)
+        return out_f, out
+
     def render_device(self, d_ptr: int, stream: int | None = None):
         """Asynchronous render of this rank's tiles into device memory (tile order)."""
         self.ctx._check(self.ctx.lib.wrt_render_device(self.ctx.h, d_ptr, stream))
