@@ -20,18 +20,11 @@ scene = Scene.from_workdir(wd, name)
 
 KNOBS = [
     ("*default", {}),
-    ("side_blocks=5", {"WRT_SIDE_BLOCKS": "5"}),
-    ("*side_blocks=6", {"WRT_SIDE_BLOCKS": "6"}),
-    ("side_blocks=7", {"WRT_SIDE_BLOCKS": "7"}),
-    ("side_blocks=8", {"WRT_SIDE_BLOCKS": "8"}),
-    ("side_blocks=6 deep_split=7", {"WRT_SIDE_BLOCKS": "6", "WRT_DEEP_SPLIT": "7"}),
-    ("side_blocks=6 deep_split=8", {"WRT_SIDE_BLOCKS": "6", "WRT_DEEP_SPLIT": "8"}),
-    ("side_blocks=6 deep_split=6", {"WRT_SIDE_BLOCKS": "6", "WRT_DEEP_SPLIT": "6"}),
-    ("side_blocks=6 deep_split=4", {"WRT_SIDE_BLOCKS": "6", "WRT_DEEP_SPLIT": "4"}),
+    ("deep_split=4", {"WRT_DEEP_SPLIT": "4"}),
+    ("deep_split=6", {"WRT_DEEP_SPLIT": "6"}),
     ("deep_split=7", {"WRT_DEEP_SPLIT": "7"}),
     ("deep_split=8", {"WRT_DEEP_SPLIT": "8"}),
-    ("side_blocks=6 refill=24", {"WRT_SIDE_BLOCKS": "6", "WRT_REFILL": "24"}),
-    ("side_blocks=6 shade0_separate=0", {"WRT_SIDE_BLOCKS": "6", "WRT_SHADE0_SEPARATE": "0"}),
+    ("shade0_separate=0", {"WRT_SHADE0_SEPARATE": "0"}),
     ("default (again)", {}),
 ]
 if os.environ.get("SWEEP_KNOBS"):             # "label:K=V,K=V;label2:..." replaces the table above

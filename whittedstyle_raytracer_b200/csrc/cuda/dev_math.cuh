@@ -49,7 +49,6 @@ __device__ __forceinline__ float4 ldg4(const float4* p) { return __ldg(p); }
 // p must be 32-byte aligned.  Divergent lanes cost the L1 one wavefront per lane and instruction, so a record fetched
 // as one 256-bit load costs half the wavefronts of two 128-bit loads (the deep closest-hit levels ran the L1 data
 // pipe at 82-87 % of its wavefront peak, profiles/NOTES.md).
-#ifndef WRT_NO_LDG256
 __device__ __forceinline__ void ldg8(const float4* p, float4& a, float4& b) {
     unsigned long long q0, q1, q2, q3;
     asm("ld.global.nc.v4.b64 {%0,%1,%2,%3}, [%4];" : "=l"(q0), "=l"(q1), "=l"(q2), "=l"(q3) : "l"(p));
@@ -58,8 +57,5 @@ __device__ __forceinline__ void ldg8(const float4* p, float4& a, float4& b) {
     b.x = __uint_as_float((unsigned)q2); b.y = __uint_as_float((unsigned)(q2 >> 32));
     b.z = __uint_as_float((unsigned)q3); b.w = __uint_as_float((unsigned)(q3 >> 32));
 }
-#else
-__device__ __forceinline__ void ldg8(const float4* p, float4& a, float4& b) { a = __ldg(p); b = __ldg(p + 1); }
-#endif
 
 } // namespace wrt

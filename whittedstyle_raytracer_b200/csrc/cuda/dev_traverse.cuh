@@ -217,9 +217,6 @@ __device__ __forceinline__ bool traverse_step(const float4* __restrict__ nodes, 
         bool right_first = NEAR_FIRST && (tr < tl);
         int far_link = right_first ? linkL : linkR;
         st.push(far_link);
-#ifdef WRT_PREFETCH_FAR
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(nodes + 2 * far_link));   // it will be popped later
-#endif
         cur = right_first ? linkR : linkL;
         return true;
     }
@@ -230,79 +227,18 @@ __device__ __forceinline__ bool traverse_step(const float4* __restrict__ nodes, 
     return true;
 }
 
-// One step over a 4-wide node (wide_bvh.h): the four grandchild records of pair `cur` in one 128-byte block.  Same
-// contract as traverse_step on a presorted octant copy; hit leaves are handled in ONE loop (one copy of the intersection
-// code, entered by every lane of the warp that has a leaf to test), inner hits are visited nearest first (NEAR_FIRST)
-// or in slot order.
-#ifndef WRT_WIDE4
-#define WRT_WIDE4 1
-#endif
-template <bool NEAR_FIRST, class LeafFn>
-__device__ __forceinline__ bool traverse_step4(const float4* __restrict__ wnodes, const Ray& r, Stack& st, int& cur,
-                                               const float& limit, LeafFn&& leaf) {
-    const float4* n = wnodes + WRT_WIDE_FLOAT4_PER_RECORD * (size_t)cur;
-    float4 a0, a1, b0, b1, c0, c1, d0, d1;
-    ldg8(n, a0, a1);
-    ldg8(n + 2, b0, b1);
-    ldg8(n + 4, c0, c1);
-    ldg8(n + 6, d0, d1);
-    float t0, t1, t2, t3;
-    bool h0 = slab_presorted(a0, a1, r, t0), h1 = slab_presorted(b0, b1, r, t1);
-    bool h2 = slab_presorted(c0, c1, r, t2), h3 = slab_presorted(d0, d1, r, t3);
-    int l0 = __float_as_int(a0.w), l1 = __float_as_int(b0.w), l2 = __float_as_int(c0.w), l3 = __float_as_int(d0.w);
-    h0 = h0 && !(t0 > limit); h1 = h1 && !(t1 > limit); h2 = h2 && !(t2 > limit); h3 = h3 && !(t3 > limit);
-    unsigned leaves = (h0 && l0 < 0 ? 1u : 0u) | (h1 && l1 < 0 ? 2u : 0u) | (h2 && l2 < 0 ? 4u : 0u) | (h3 && l3 < 0 ? 8u : 0u);
-    while (leaves) {
-        const unsigned j = __ffs(leaves) - 1;
-        leaves &= leaves - 1;
-        const int lk = j == 0 ? l0 : (j == 1 ? l1 : (j == 2 ? l2 : l3));
-        const float tj = j == 0 ? t0 : (j == 1 ? t1 : (j == 2 ? t2 : t3));
-        if (!(tj > limit)) leaf(~lk);                      // `limit` may have tightened in an earlier leaf()
-    }
-    const float inf = INFINITY;
-    // inner hits: key = entry distance, +inf = not to be visited
-    float k0 = (h0 && l0 >= 0 && !(t0 > limit)) ? t0 : inf, k1 = (h1 && l1 >= 0 && !(t1 > limit)) ? t1 : inf;
-    float k2 = (h2 && l2 >= 0 && !(t2 > limit)) ? t2 : inf, k3 = (h3 && l3 >= 0 && !(t3 > limit)) ? t3 : inf;
-    if (NEAR_FIRST) {
-#define WRT_CSWAP(ka, la, kb, lb) { const bool sw = kb < ka; const float kt = sw ? ka : kb; ka = sw ? kb : ka; kb = kt; const int lt = sw ? la : lb; la = sw ? lb : la; lb = lt; }
-        WRT_CSWAP(k0, l0, k1, l1) WRT_CSWAP(k2, l2, k3, l3) WRT_CSWAP(k0, l0, k2, l2) WRT_CSWAP(k1, l1, k3, l3) WRT_CSWAP(k1, l1, k2, l2)
-#undef WRT_CSWAP
-        if (k0 < inf) {                                    // ascending: (k0,l0) nearest
-            if (k3 < inf) st.push(l3);
-            if (k2 < inf) st.push(l2);
-            if (k1 < inf) st.push(l1);
-            cur = l0;
-            return true;
-        }
-    } else {
-        int nxt = -1;
-        if (k0 < inf) nxt = l0;
-        if (k1 < inf) { if (nxt >= 0) st.push(nxt); nxt = l1; }
-        if (k2 < inf) { if (nxt >= 0) st.push(nxt); nxt = l2; }
-        if (k3 < inf) { if (nxt >= 0) st.push(nxt); nxt = l3; }
-        if (nxt >= 0) { cur = nxt; return true; }
-    }
-    if (st.empty()) return false;
-    cur = st.pop();
-    return true;
-}
-
-// The closest-hit walk over the 4-wide view with DEFERRED leaves.  traverse_step4 tests every hit leaf of a node at once:
-// a lane with two leaf hits runs the ~110-instruction intersection code twice while the warp's other lanes wait, and in a
-// warp of ~24 walking lanes some lane has a second leaf in nearly every step — so the warp pays two or three rounds of
-// leaf code per node step, the later ones with 2-3 lanes.  Here a lane tests at most ONE leaf per step, at one code site:
-// of a node's hits, taken nearest first, the first leaf goes to the lane's leaf slot, the first other hit becomes `cur`
-// (an inner pair, or a leaf link: it is then tested by the next step), the rest is pushed far to near — leaf links (< 0)
-// lie on the stack beside pair indices.  A step whose `cur` is a leaf link takes it into the leaf slot and visits the
-// pair on top of the stack beside it.  Exactness: every tested primitive has had its own box hit by the ray, and the
-// closest-hit result (min t, ties to the smaller primitive index) does not depend on the order of the tests; a deferred
-// leaf is tested without its entry distance (a superset of what the pruning keeps).
-#ifndef WRT_LEAF_DEFER
-#define WRT_LEAF_DEFER 2           // 0: traverse_step4 everywhere; 1: deferred leaves in the closest-hit walk; 2: and in the hard-shadow walk
-#endif
-#ifndef WRT_LEAF_DEFER_SIMPLE
-#define WRT_LEAF_DEFER_SIMPLE 1
-#endif
+// One step over a 4-wide node (wide_bvh.h): the four grandchild records of pair `cur` in one 128-byte block, on a
+// presorted octant copy, with DEFERRED leaves.  Testing every hit leaf of a node at once, a lane with two leaf hits runs
+// the ~110-instruction intersection code twice while the warp's other lanes wait, and in a warp of ~24 walking lanes
+// some lane has a second leaf in nearly every step — so the warp pays two or three rounds of leaf code per node step, the
+// later ones with 2-3 lanes.  Here a lane tests at most ONE leaf per step, at one code site: of a node's hits, taken
+// nearest first (NEAR_FIRST: the closest-hit walk) or in slot order (the hard-shadow walk), the first leaf goes to the
+// lane's leaf slot, the first other hit becomes `cur` (an inner pair, or a leaf link: it is then tested by the next
+// step), the rest is pushed far to near — leaf links (< 0) lie on the stack beside pair indices.  A step whose `cur` is
+// a leaf link takes it into the leaf slot and visits the pair on top of the stack beside it.  Exactness: every tested
+// primitive has had its own box hit by the ray, and the closest-hit result (min t, ties to the smaller primitive index)
+// does not depend on the order of the tests; a deferred leaf is tested without its entry distance (a superset of what the
+// pruning keeps).
 #define WRT_NO_LINK (-2147483647 - 1)      // (also the link of a wide node's empty slot, which no ray reaches)
 template <bool NEAR_FIRST, class LeafFn>
 __device__ __forceinline__ bool traverse_step4_defer(const float4* __restrict__ wnodes, const Ray& r, Stack& st, int& cur,
@@ -334,7 +270,6 @@ __device__ __forceinline__ bool traverse_step4_defer(const float4* __restrict__ 
 #define WRT_CSWAP(ka, la, kb, lb) { const bool sw = kb < ka; const float kt = sw ? ka : kb; ka = sw ? kb : ka; kb = kt; const int lt = sw ? la : lb; la = sw ? lb : la; lb = lt; }
         if (NEAR_FIRST) { WRT_CSWAP(k0, l0, k1, l1) WRT_CSWAP(k2, l2, k3, l3) WRT_CSWAP(k0, l0, k2, l2) WRT_CSWAP(k1, l1, k3, l3) WRT_CSWAP(k1, l1, k2, l2) }
 #undef WRT_CSWAP
-#if WRT_LEAF_DEFER_SIMPLE
         if (NEAR_FIRST) {
             // sorted: the hits are k0 <= k1 <= ..., misses (+inf) last.  Only the NEAREST hit may go to the leaf slot; a leaf
             // further back becomes `cur` or waits on the stack like a pair (a third of the bookkeeping instructions of the
@@ -348,25 +283,22 @@ __device__ __forceinline__ bool traverse_step4_defer(const float4* __restrict__ 
             if (k2 < inf) st.push(l2);
             if (!tk && k1 < inf) st.push(l1);
         } else {
-#else
-        {
-#endif
-        bool have_p = pend != WRT_NO_LINK, have_c = false;
-        cur = WRT_NO_LINK;
-        // nearest first: leaf slot, then `cur`, the others wait on the stack
+            bool have_p = pend != WRT_NO_LINK, have_c = false;
+            cur = WRT_NO_LINK;
+            // in slot order: leaf slot, then `cur`, the others wait on the stack
 #define WRT_TAKE(kj, lj, pushj)                                                                    \
-        bool pushj = false;                                                                        \
-        if (kj < inf) {                                                                            \
-            if (lj < 0 && !have_p) { pend = lj; tp = kj; have_p = true; }                          \
-            else if (!have_c) { cur = lj; have_c = true; }                                         \
-            else pushj = true;                                                                     \
-        }
-        WRT_TAKE(k0, l0, p0) WRT_TAKE(k1, l1, p1) WRT_TAKE(k2, l2, p2) WRT_TAKE(k3, l3, p3)
+            bool pushj = false;                                                                    \
+            if (kj < inf) {                                                                        \
+                if (lj < 0 && !have_p) { pend = lj; tp = kj; have_p = true; }                      \
+                else if (!have_c) { cur = lj; have_c = true; }                                     \
+                else pushj = true;                                                                 \
+            }
+            WRT_TAKE(k0, l0, p0) WRT_TAKE(k1, l1, p1) WRT_TAKE(k2, l2, p2) WRT_TAKE(k3, l3, p3)
 #undef WRT_TAKE
-        (void)p0;                                          // the nearest hit always finds a free place
-        if (p3) st.push(l3);
-        if (p2) st.push(l2);
-        if (p1) st.push(l1);
+            (void)p0;                                          // the first hit always finds a free place
+            if (p3) st.push(l3);
+            if (p2) st.push(l2);
+            if (p1) st.push(l1);
         }
     }
     // (Taking the next node from the stack BEFORE the leaf test and prefetching its line to L1 meanwhile: closest hit 3.68 ->
@@ -653,12 +585,8 @@ __device__ __forceinline__ float directional_product_bvh(const DevScene& s, cons
 //             bool step(cur, st)         — one traversal step; false = finished
 //             bool finish(cur, st)       — a walk ended: write results, or start the item's next
 //                                          walk and return true
-#ifndef WRT_STEPS_PER_ROUND
 #define WRT_STEPS_PER_ROUND 4      // traversal steps between two looks at the warp's idle lanes (the deep closest-hit levels: 8)
-#endif
-#ifndef WRT_CHUNK_MIN_PER
 #define WRT_CHUNK_MIN_PER 256
-#endif
 
 template <class Q, int STEPS = WRT_STEPS_PER_ROUND>
 __device__ __forceinline__ void run_queue(Q& q, unsigned long long n, unsigned long long* work, Stack& st, int refill_cfg) {

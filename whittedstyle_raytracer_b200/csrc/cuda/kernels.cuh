@@ -36,14 +36,8 @@
 
 // Traversal kernels: 128-thread CTAs; ptxas settles at 48-61 registers (8-9 CTAs per SM).  Forcing more
 // CTAs per SM through a minimum-blocks bound spills and is slower (profiles/NOTES.md).
-#ifdef WRT_MIN_BLOCKS
-#define WRT_TRACE_BOUNDS __launch_bounds__(128, WRT_MIN_BLOCKS)
-#else
 #define WRT_TRACE_BOUNDS __launch_bounds__(128)
-#endif
-#ifndef WRT_TRACE_DEEP_STEPS
 #define WRT_TRACE_DEEP_STEPS 8
-#endif
 namespace wrt {
 
 // ---- debug build (-DWRT_DEBUG_BOUNDS): every queue / pool / stack / node index is checked before the access; the first
@@ -383,7 +377,7 @@ struct ClosestQuery {
         if (cur < 0) { cs.leaf(s, r, ~cur); return false; }
         // (level 0: coherent primary rays, two thirds of them end on a wall after a few steps — the 4-wide node costs
         // registers there and buys nothing: 378 vs 338 us)
-        wide = WRT_WIDE4 && !LEVEL0 && !ref_tree;
+        wide = !LEVEL0 && !ref_tree;
         // (One copy for all octants — octant 0's holds the plain {pMin}{pMax} records — with the select-based slab test, to
         // shrink the L1 footprint of the deep levels 8x: 3.73 against 3.70 ms, no gain; the fetches that stall are L2 hits
         // deep in the tree, not the shared top levels.)
@@ -391,11 +385,7 @@ struct ClosestQuery {
         return true;
     }
     __device__ __forceinline__ bool step(int& cur, Stack& st) {
-#if WRT_LEAF_DEFER
-        if (WRT_WIDE4 && !LEVEL0 && wide) return traverse_step4_defer<true>(nodes, r, st, cur, cs.limit, [&](int p) { cs.leaf(s, r, p); });
-#else
-        if (WRT_WIDE4 && !LEVEL0 && wide) return traverse_step4<true>(nodes, r, st, cur, cs.limit, [&](int p) { cs.leaf(s, r, p); });
-#endif
+        if (!LEVEL0 && wide) return traverse_step4_defer<true>(nodes, r, st, cur, cs.limit, [&](int p) { cs.leaf(s, r, p); });
         return traverse_step<true, true>(nodes, r, st, cur, cs.limit, [&](int p) { cs.leaf(s, r, p); });
     }
     __device__ __forceinline__ bool finish(int&, Stack&) {
@@ -421,9 +411,7 @@ __global__ void WRT_TRACE_BOUNDS k_trace_closest(const __grid_constant__ DevScen
 // ---- K3: hit -> surface, shadow requests, child rays: one streaming pass, whole warps call surface_warp() ----
 // (launch bound: 64 registers = 4 CTAs of 256 per SM.  Unbounded the kernel takes 80 registers, 3 CTAs: 1.67 ms per 4K
 // frame against 1.61 / hard-shadow frame 1.72 against 1.36; 5 CTAs (48 registers) spill too much: 1.97.)
-#ifndef WRT_SURFACE_MIN_BLOCKS
 #define WRT_SURFACE_MIN_BLOCKS 4
-#endif
 __global__ void __launch_bounds__(256, WRT_SURFACE_MIN_BLOCKS) k_surface_spawn(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
                                                        const __grid_constant__ PrimaryGen pg, int level, unsigned n0, int cull) {
     const LevelSpan span = level_span(fb, level, n0);
@@ -489,18 +477,14 @@ struct HardShadowQuery {
         if (!slab_presorted(lo, hi, r, te)) return false;
         cur = __float_as_int(lo.w);
         if (cur < 0) { shadow_leaf(s, r, dis, ~cur, acc); return false; }
-        wide = WRT_WIDE4 && !ref_tree;
+        wide = !ref_tree;
         if (wide) nodes = s.wnodes + (WRT_WIDE_FLOAT4_PER_RECORD / 2) * oct_off;
         return true;
     }
     __device__ __forceinline__ bool step(int& cur, Stack& st) {
         const float never = INFINITY;
         bool more;
-#if WRT_LEAF_DEFER >= 2
-        if (WRT_WIDE4 && wide) more = traverse_step4_defer<false>(nodes, r, st, cur, never, [&](int p) { shadow_leaf(s, r, dis, p, acc); });
-#else
-        if (WRT_WIDE4 && wide) more = traverse_step4<false>(nodes, r, st, cur, never, [&](int p) { shadow_leaf(s, r, dis, p, acc); });
-#endif
+        if (wide) more = traverse_step4_defer<false>(nodes, r, st, cur, never, [&](int p) { shadow_leaf(s, r, dis, p, acc); });
         else more = traverse_step<false, true>(nodes, r, st, cur, never, [&](int p) { shadow_leaf(s, r, dis, p, acc); });
         return more && acc.res != 0.f;
     }
@@ -624,40 +608,31 @@ __global__ void WRT_TRACE_BOUNDS k_shadow_soft(const __grid_constant__ DevScene 
 #endif
 struct SoftListBuffers {
     int*  scratch;        // WRT_LIST_CAP ints per thread of the grid: a walk writes here, then copies into the pool
-    float* shafts;        // WRT_LISTS_CHUNK x WRT_SHAFT_SLOT floats per warp of the grid: the shafts of the warp's current chunk
+    float* shafts;        // WRT_LISTS_CHUNK x WRT_SHAFT_SLOT floats per warp of the grid: the warp's ring of prepared shafts
     int*  pool;           // the lists
     int2* ref;            // per request: {pool offset, count}
     unsigned* work;       // k_soft_filter: the requests that need rays (non-empty list, or count < 0), compacted
     unsigned pool_cap;
-    unsigned region_per_request;   // pool entries a warp reserves per request of its chunk (one atomic per chunk)
 };
-#ifndef WRT_LIST_TRI_FIRST
-#define WRT_LIST_TRI_FIRST 1
-#endif
-#ifndef WRT_LIST_CHUNK_PASSES
 #define WRT_LIST_CHUNK_PASSES 8
-#endif
-#ifndef WRT_LISTS_CHUNK
 #define WRT_LISTS_CHUNK 128
-#endif
-#ifndef WRT_LISTS_REFILL
 #define WRT_LISTS_REFILL 8
-#endif
 #define WRT_SHAFT_SLOT 12         // floats a staged shaft occupies: o, ilo, ihi, octant | use, -, request index
 
 // One lane walks one request's shaft, but walk lengths differ a lot (3 ... 400 node pairs; ncu: 8.6 of 32 lanes
-// active when every lane takes one request and the warp waits for the longest).  So a warp owns a chunk of
-// consecutive requests at a time (32 ... WRT_LISTS_CHUNK, by queue length):
-//   A. all lanes build the chunk's shafts (wrt_shaft_make, ~200 instructions, fully converged) into a per-warp slot
-//      array (global scratch, L1-resident);
-//   B. lanes walk; a finished lane keeps its list in its scratch column and goes idle; once WRT_LISTS_REFILL lanes are
-//      idle the WHOLE warp flushes the finished lists into the pool (coalesced copies, 32 entries per step — a lane
-//      copying its own list alone stalls the other 31: measured, 27 % slower than no refill at all) and hands the
-//      chunk's next requests to the idle lanes (a slot load, no set-up code on a few lanes).
-// Pool space: the warp reserves region_per_request entries per request of the chunk with ONE global atomic and
-// allocates from the region through a warp-uniform cursor; when the region is used up it takes what the flush needs
-// with another atomic; an exhausted pool means count = -1 (per-ray walk).  Lists of a chunk stay close together.
-// (An earlier refill attempt through run_queue — set-up code on the refilled lanes only — was slower than no refill.)
+// active when every lane takes one request and the warp waits for the longest).  So a finished lane keeps its list in its
+// scratch column and goes idle; whenever WRT_LISTS_REFILL lanes are idle the WHOLE warp flushes the finished lists into the
+// pool (coalesced copies, 32 entries per step — a lane copying its own list alone stalls the other 31: measured, 27 %
+// slower than no refill at all) and hands the idle lanes new requests from a small ring of PREPARED requests, a per-warp
+// slot array (global scratch, L1-resident).  All lanes build the ring's shafts (wrt_shaft_make, ~200 instructions, fully
+// converged — set-up code on a few lanes at a time is what made a refill through run_queue slower than no refill at
+// all), 32 requests per claim from the global counter, whenever the idle lanes outnumber the prepared requests.  A lane
+// keeps the index of its request in a register: its ring slot may be reused while it is still walking.  Pool space is
+// taken per flush (>= WRT_LISTS_REFILL lists, one atomic); an exhausted pool means count = -1 (per-ray walk).
+// (A chunked form — a warp owns up to 128 consecutive requests, walks them all, then claims the next chunk — ends every
+// chunk with its longest walk: on a short queue (one GPU's share of an 8-GPU frame: 2-3 requests per lane) a chunk is one
+// request per lane, almost every chunk holds a request in shadow whose walk is 5x the average, and the lanes wait for it:
+// 695 us for 0.5 M requests where the work is ~150 us.)
 // (launch bound, with the 4-wide walk: 8 CTAs per SM = 63 registers, no spills: 2.86 ms per 4K frame; 10 CTAs = 48 registers,
 // 24 bytes of spills: 3.13 ms; unbounded 80 registers: 5 CTAs.)
 // (A per-leaf "own plane" test inside the walk — three quarters of the leaves a fully lit request finds are its own
@@ -665,20 +640,7 @@ struct SoftListBuffers {
 // costs two dependent loads and ~40 instructions at that width: 6.3 ms against 3.1.  The same test a candidate per lane
 // while the warp copies a finished list into the pool: 3.7 ms against 2.6 — the flush is the serial part of this kernel.
 // The filter kernel, which spreads (request, candidate) pairs over all lanes, is the right place.)
-#ifndef WRT_LISTS_MIN_BLOCKS
 #define WRT_LISTS_MIN_BLOCKS 8
-#endif
-#ifndef WRT_LISTS_STREAM
-#define WRT_LISTS_STREAM 1        // 1: a warp claims 32 requests whenever its idle lanes outnumber the prepared requests
-#endif
-#if WRT_LISTS_STREAM
-// Streaming form.  The chunked form below ends every chunk with its longest walk: on a short queue (one GPU's share of an
-// 8-GPU frame: 2-3 requests per lane) a chunk is one request per lane, almost every chunk holds a request in shadow whose
-// walk is 5x the average, and the lanes wait for it: 695 us for 0.5 M requests where the work is ~150 us.  Here a warp never
-// waits for a chunk: whenever WRT_LISTS_REFILL lanes are idle it flushes their lists and hands them new requests from a
-// small ring of PREPARED requests (shafts built 32 at a time by all lanes, fully converged — set-up code on a few lanes
-// at a time is what made the run_queue attempt slower); the ring is topped up from the global counter, 32 requests per
-// claim.  A lane keeps the index of its request in a register: its ring slot may be reused while it is still walking.  Pool space is taken per flush (>= WRT_LISTS_REFILL lists, one atomic).
 __global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb, int q,
                                                         int work_slot, int stack_rows, SoftListBuffers lb) {
     extern __shared__ int smem[];
@@ -785,11 +747,7 @@ __global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const 
                         sh.ilo[0] = d[3]; sh.ilo[1] = d[4]; sh.ilo[2] = d[5];
                         sh.ihi[0] = d[6]; sh.ihi[1] = d[7]; sh.ihi[2] = d[8];
                         sh.octant = ou & 7; sh.use = ou >> 3;
-#if WRT_WIDE4
                         rc = wrt_shaft_walk_begin4(s.onodes, s.wnodes, s.n_nodes, &sh, &w);
-#else
-                        rc = wrt_shaft_walk_begin(s.onodes, s.n_nodes, &sh, &w);
-#endif
                     }
                     if (rc == 1) active = true;
                     else pend = rc;                          // answered without a walk; recorded by the next flush
@@ -805,11 +763,7 @@ __global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const 
 #pragma unroll 1
         for (int it = 0; it < 4; it++) {
             if (active) {
-#if WRT_WIDE4
                 const int rc = wrt_shaft_walk_step4(&sh, &w, st.base, st.stride, stack_rows, mine, WRT_LIST_CAP);
-#else
-                const int rc = wrt_shaft_walk_step(&sh, &w, st.base, st.stride, stack_rows, mine, WRT_LIST_CAP);
-#endif
                 if (rc != 1) { active = false; pend = rc < 0 ? -1 : w.n; }
             }
         }
@@ -817,165 +771,6 @@ __global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const 
     n_empty = __reduce_add_sync(0xffffffffu, n_empty);
     if (lane == 0 && n_empty) atomicAdd(fb.counters + C_NEMPTY, n_empty);
 }
-#else
-__global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb, int q,
-                                                        int work_slot, int stack_rows, SoftListBuffers lb) {
-    extern __shared__ int smem[];
-    Stack st;
-    st.init(smem, threadIdx.x, blockDim.x);
-    const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const unsigned lt_mask = (1u << lane) - 1u;
-    const unsigned nreq = queue_len(fb.counters, C_NPREQ + q, fb.preq_cap[q]);
-    const size_t gwarp = (size_t)blockIdx.x * (blockDim.x >> 5) + warp;
-    int* warp_scratch = lb.scratch + gwarp * 32 * WRT_LIST_CAP;
-    int* mine = warp_scratch + (size_t)lane * WRT_LIST_CAP;
-    float* slots = lb.shafts + gwarp * (size_t)WRT_LISTS_CHUNK * WRT_SHAFT_SLOT;
-    unsigned long long* work = reinterpret_cast<unsigned long long*>(fb.counters + work_slot);
-    unsigned* pool_head = fb.counters + C_POOL + q;
-    // chunk size: ~4 chunks per warp on short queues (the launch ends with its slowest chunk), WRT_LISTS_CHUNK on long ones
-    unsigned chunk_size;
-    {
-        const unsigned long long warps = (unsigned long long)gridDim.x * (blockDim.x >> 5);
-        unsigned long long per = nreq / (warps * 4ull);
-        per = (per + 31ull) & ~31ull;
-        chunk_size = per < 32ull ? 32u : (per > (unsigned long long)WRT_LISTS_CHUNK ? (unsigned)WRT_LISTS_CHUNK : (unsigned)per);
-    }
-    unsigned n_empty = 0;
-    while (true) {
-        unsigned long long claimed = 0;
-        if (lane == 0) claimed = atomicAdd(work, (unsigned long long)chunk_size);
-        claimed = __shfl_sync(0xffffffffu, claimed, 0);
-        if (claimed >= nreq) break;
-        const unsigned base = (unsigned)claimed;
-        const unsigned chunk = nreq - base < chunk_size ? nreq - base : chunk_size;
-        // ---- A: shafts of the chunk ----
-        for (unsigned r = lane; r < chunk; r += 32) {
-            float4 o4 = fb.preq_o[q][base + r];
-            uint4 k = fb.preq_k[q][base + r];
-            const WrtLight* L = s.lights + k.x;
-            float tri[9];
-            for (int i = 0; i < 9; i++) tri[i] = L->tri[i];
-            const float o[3] = {o4.x, o4.y, o4.z};
-            WrtShaft sh;
-            const bool ok = wrt_shaft_make(o, tri, &sh);
-            float* d = slots + (size_t)r * WRT_SHAFT_SLOT;
-            d[0] = sh.o[0]; d[1] = sh.o[1]; d[2] = sh.o[2];
-            d[3] = sh.ilo[0]; d[4] = sh.ilo[1]; d[5] = sh.ilo[2];
-            d[6] = sh.ihi[0]; d[7] = sh.ihi[1]; d[8] = sh.ihi[2];
-            d[9] = __int_as_float(ok ? (sh.octant | (sh.use << 3)) : -1);
-            d[10] = 0.f;
-            d[11] = __uint_as_float(k.x);
-        }
-        // ---- pool region of the chunk: one atomic; [cursor, region_end) is what is left of it (warp-uniform) ----
-        unsigned cursor = 0;
-        if (lane == 0) cursor = atomicAdd(pool_head, chunk * lb.region_per_request);
-        cursor = __shfl_sync(0xffffffffu, cursor, 0);
-        unsigned region_end = cursor + chunk * lb.region_per_request;
-        if (cursor >= lb.pool_cap) { cursor = 0; region_end = 0; }
-        else if (region_end > lb.pool_cap || region_end < cursor) region_end = lb.pool_cap;
-        __syncwarp();
-        // ---- B: walks, flush + refill ----
-        unsigned next = 0;                                   // warp-uniform: requests of the chunk handed out so far
-        bool active = false;
-        int pend = -2;                                       // finished walk waiting for the flush: list length, -1 = give up; -2 = nothing
-        unsigned my = 0;
-        WrtShaft sh;
-        WrtShaftWalk w;
-        w.nodes = s.onodes; w.cur = 0; w.sp = 0; w.n = 0;
-        while (true) {
-            const unsigned idle = __ballot_sync(0xffffffffu, !active);
-            const bool more = next < chunk;
-            if (idle == 0xffffffffu || (more && __popc(idle) >= WRT_LISTS_REFILL)) {
-                // flush: the finished lists -> pool, all lanes copying
-                __syncwarp();                                // the lists other lanes wrote to their scratch columns are visible
-                const int cnt = pend > 0 ? pend : 0;
-                int incl = cnt;
-#pragma unroll
-                for (int off = 1; off < 32; off <<= 1) {
-                    int v = __shfl_up_sync(0xffffffffu, incl, off);
-                    if (lane >= (unsigned)off) incl += v;
-                }
-                const unsigned total = (unsigned)__shfl_sync(0xffffffffu, incl, 31);
-                if (total > 0) {
-                    unsigned first = cursor;
-                    bool fits = total <= region_end - cursor;
-                    if (fits) cursor += total;
-                    else {                                   // region used up: take exactly what this flush needs
-                        unsigned g = 0xffffffffu;
-                        if (lane == 0 && *(volatile unsigned*)pool_head < lb.pool_cap) g = atomicAdd(pool_head, total);
-                        g = __shfl_sync(0xffffffffu, g, 0);
-                        fits = g < lb.pool_cap && total <= lb.pool_cap - g;
-                        first = g;
-                    }
-                    const unsigned dst = first + (unsigned)(incl - cnt);
-                    unsigned todo = __ballot_sync(0xffffffffu, cnt > 0);
-                        while (todo) {
-                        const int src_lane = __ffs(todo) - 1;
-                        todo &= todo - 1;
-                        const int c = __shfl_sync(0xffffffffu, cnt, src_lane);
-                        const unsigned d0 = __shfl_sync(0xffffffffu, dst, src_lane);
-                        if (fits) {
-                            const int* src = warp_scratch + (size_t)src_lane * WRT_LIST_CAP;
-                            for (int i = (int)lane; i < c; i += 32)
-                                if (WRT_IN_BOUNDS(d0 + i, lb.pool_cap)) lb.pool[d0 + i] = src[i];
-                        }
-                    }
-                    if (cnt > 0 && WRT_IN_BOUNDS(base + my, fb.preq_cap[q])) lb.ref[base + my] = fits ? make_int2((int)dst, cnt) : make_int2(0, -1);
-                }
-                if (pend == 0 || pend == -1) {               // empty list (= lit, no rays needed) / give up (= ray by ray)
-                    if (WRT_IN_BOUNDS(base + my, fb.preq_cap[q])) lb.ref[base + my] = make_int2(0, pend);
-                    if (pend == 0) ++n_empty;
-                }
-                pend = -2;
-                __syncwarp();                                // the scratch columns are free again
-                // refill
-                if (more) {
-                    const unsigned cand = next + __popc(idle & lt_mask);
-                    next += __popc(idle);
-                    if (!active && cand < chunk) {
-                        my = cand;
-                        const float* d = slots + (size_t)my * WRT_SHAFT_SLOT;
-                        const int ou = __float_as_int(d[9]);
-                        int rc = -1;
-                        if (ou >= 0) {
-                            sh.o[0] = d[0]; sh.o[1] = d[1]; sh.o[2] = d[2];
-                            sh.ilo[0] = d[3]; sh.ilo[1] = d[4]; sh.ilo[2] = d[5];
-                            sh.ihi[0] = d[6]; sh.ihi[1] = d[7]; sh.ihi[2] = d[8];
-                            sh.octant = ou & 7; sh.use = ou >> 3;
-#if WRT_WIDE4
-                            rc = wrt_shaft_walk_begin4(s.onodes, s.wnodes, s.n_nodes, &sh, &w);
-#else
-                            rc = wrt_shaft_walk_begin(s.onodes, s.n_nodes, &sh, &w);
-#endif
-                        }
-                        if (rc == 1) active = true;
-                        else pend = rc;                      // answered without a walk; recorded by the next flush
-                    }
-                }
-                if (!__any_sync(0xffffffffu, active)) {
-                    if (next >= chunk && !__any_sync(0xffffffffu, pend != -2)) break;
-                    continue;
-                }
-            }
-#pragma unroll 1
-            for (int it = 0; it < 4; it++) {
-                if (active) {
-#if WRT_WIDE4
-                    const int rc = wrt_shaft_walk_step4(&sh, &w, st.base, st.stride, stack_rows, mine, WRT_LIST_CAP);
-#else
-                    const int rc = wrt_shaft_walk_step(&sh, &w, st.base, st.stride, stack_rows, mine, WRT_LIST_CAP);
-#endif
-                    if (rc != 1) { active = false; pend = rc < 0 ? -1 : w.n; }
-                }
-            }
-        }
-        __syncwarp();
-    }
-    n_empty = __reduce_add_sync(0xffffffffu, n_empty);
-    if (lane == 0 && n_empty) atomicAdd(fb.counters + C_NEMPTY, n_empty);
-}
-
-#endif
 
 // ---- K4b'': triangle-level pruning of the candidate lists (shaft_cull.h, wrt_pyramid_*) ----
 // The lists hold every primitive whose BOX a ray of the shaft may hit.  On the bunny's surface half of those triangles
@@ -984,10 +779,8 @@ __global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const 
 // per request drops them (ballot compaction, in place, order kept).  A quarter of the fully lit deep requests end up
 // with an empty list and need no rays at all.  Exact: a removed triangle blocks no sample ray (proof obligations and the
 // brute-force check: shaft_cull.h, tests/shaft_cull_check.cpp).
-#ifndef WRT_FILTER_MIN
 #define WRT_FILTER_MIN 1          // every non-empty list: with the edge planes most 1- and 2-member lists of fully lit requests
                                   // come out empty and their 50 rays are never built (3 / 2 / 1: 14.19 / 13.64 / 13.57 ms per 4K frame)
-#endif
 // A warp takes 32 consecutive requests: (A) each lane builds its request's pyramid (4 cross products, 8 square roots, 4
 // divisions — once per request, not once per candidate) into shared memory; (B) the 32 lists are treated as ONE sequence
 // of (request, candidate) pairs, 32 pairs per step, one per lane: most lists of fully lit requests hold 1-4 candidates, and
@@ -998,9 +791,7 @@ __global__ void __launch_bounds__(128, WRT_LISTS_MIN_BLOCKS) k_soft_lists(const 
 // kept: rank = kept-so-far of the request (shared memory) + survivors of the same request on lower lanes
 // (__match_any_sync).  A request's write cursor never passes its read cursor, and every step reads before it writes.
 // (no minimum-blocks bound: the pyramid spills under one)
-#ifndef WRT_FILTER_EDGE_MAX
 #define WRT_FILTER_EDGE_MAX 16    // survivor lists up to this length get the edge-plane stage
-#endif
 // One pass of k_soft_filter over the lists of a warp's 32 requests (lane r <-> request r): kept[r] entries of list r
 // (request r takes part iff `take`), all lists as one sequence of pairs, 32 per step; survivors compacted in place.
 template <int STAGE>
@@ -1063,16 +854,11 @@ __device__ __forceinline__ void filter_pass(const DevScene& s, const SoftListBuf
     }
 }
 
-#ifndef WRT_FILTER_MIN_BLOCKS
 #define WRT_FILTER_MIN_BLOCKS 8   // 64 registers, no spills (unbounded: 70 registers, 7 CTAs per SM, 1.51 against 1.44 ms)
-#endif
 #define WRT_FILTER_BOUNDS __launch_bounds__(128, WRT_FILTER_MIN_BLOCKS)
-// Work distribution: blocks of 32 requests are claimed from a global counter (WRT_FILTER_DYNAMIC; the host sizes the grid to
-// what is resident).  The static round-robin over 8 CTAs per SM it replaces ran in two waves — 7 CTAs of 72 registers fit —
+// Work distribution: blocks of 32 requests are claimed from a global counter (the host sizes the grid to what is
+// resident).  The static round-robin over 8 CTAs per SM it replaces ran in two waves — 7 CTAs of 72 registers fit —
 // the second one with a single CTA per SM (ncu: 22-31 % achieved occupancy of 44 % possible).
-#ifndef WRT_FILTER_DYNAMIC
-#define WRT_FILTER_DYNAMIC 1
-#endif
 __global__ void WRT_FILTER_BOUNDS k_soft_filter(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb, int q,
                                                      SoftListBuffers lb, int work_slot) {
     __shared__ float s_py[4][32][WRT_PYRAMID_FLOATS + 1];
@@ -1080,11 +866,9 @@ __global__ void WRT_FILTER_BOUNDS k_soft_filter(const __grid_constant__ DevScene
     const unsigned lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const unsigned lt_mask = (1u << lane) - 1u;
     const unsigned nreq = queue_len(fb.counters, C_NPREQ + q, fb.preq_cap[q]);
-    const unsigned warps = gridDim.x * (blockDim.x >> 5), gw = blockIdx.x * (blockDim.x >> 5) + warp;
+    const unsigned warps = gridDim.x * (blockDim.x >> 5);
     unsigned n_empty = 0;
-#if WRT_FILTER_DYNAMIC
     unsigned long long* work = reinterpret_cast<unsigned long long*>(fb.counters + work_slot);
-    (void)gw;
     // requests per claim: 32 (one per lane) on a long queue; on a short one — a rank's share of a multi-GPU frame holds
     // less than a block per warp — 16 or 8, so that the launch does not end with the one warp that drew 32 long lists
     const unsigned per_claim = nreq >= warps * 64u ? 32u : (nreq >= warps * 16u ? 16u : 8u);
@@ -1095,10 +879,6 @@ __global__ void WRT_FILTER_BOUNDS k_soft_filter(const __grid_constant__ DevScene
         if (claimed >= nreq) break;
         const unsigned base = (unsigned)claimed;
         const unsigned lim = base + per_claim < nreq ? base + per_claim : nreq;    // this claim's requests end here
-#else
-    for (unsigned base = gw * 32u; base < nreq; base += warps * 32u) {
-        const unsigned lim = nreq;
-#endif
         // ---- A ----
         const unsigned req = base + lane;
         int2 ref = make_int2(0, 0);
@@ -1217,7 +997,6 @@ __global__ void WRT_TRACE_BOUNDS k_soft_list_rays(const __grid_constant__ DevSce
                     occ = occluded(s, degenerate_dir(raydir) ? s.nodes : s.fnodes, r, dis, st);
                 } else {
                     const int* list = lb.pool + ref.x;
-#if WRT_LIST_TRI_FIRST
                     // occ = OR over the list of (own box hit && intersection accepted && t < dis): the same conjunction with
                     // the intersection test first.  k_soft_filter leaves candidates that can really block, so 7 of 10 box
                     // tests pass and the warp runs the intersection code in every iteration anyway; the box test (two
@@ -1232,9 +1011,6 @@ __global__ void WRT_TRACE_BOUNDS k_soft_list_rays(const __grid_constant__ DevSce
                             occ = slab(blo, bhi, r, te);
                         }
                     }
-#else
-                    for (int c = 0; c < ref.y && !occ; c++) occ = occluder_cache_hit(s, r, dis, list[c]);
-#endif
                 }
                 lit = !occ;
             }

@@ -270,9 +270,6 @@ WRT_SHAFT_HD int wrt_shaft_walk_begin4(const float4* onodes, const float4* wnode
     return w->cur < 0 ? -1 : 1;                                           // lone primitive: tested without its box
 }
 
-#ifndef WRT_SHAFT_STEP_BRANCHFREE
-#define WRT_SHAFT_STEP_BRANCHFREE 1
-#endif
 #define WRT_SHAFT_CSWAP(ka, la, kb, lb) { const bool sw_ = (kb) < (ka); const float kt_ = sw_ ? (ka) : (kb); (ka) = sw_ ? (kb) : (ka); (kb) = kt_; \
                                           const int lt_ = sw_ ? (la) : (lb); (la) = sw_ ? (lb) : (la); (lb) = lt_; }
 
@@ -301,55 +298,36 @@ WRT_SHAFT_HD int wrt_shaft_walk_step4(const WrtShaft* sh, WrtShaftWalk* w, int* 
     WRT_SHAFT_CSWAP(k0, l0, k1, l1) WRT_SHAFT_CSWAP(k2, l2, k3, l3) WRT_SHAFT_CSWAP(k0, l0, k2, l2)
     WRT_SHAFT_CSWAP(k1, l1, k3, l3) WRT_SHAFT_CSWAP(k1, l1, k2, l2)
     int n = w->n;
-#if WRT_SHAFT_STEP_BRANCHFREE
     // Straight-line form: the capacity checks once per step (a list / stack within 4 / 3 entries of its capacity gives up a
     // step early: the request is then traced ray by ray, an exact path too), the appends and pushes as predicated stores.
-    // (ncu source view of the branching form below: 36 % of k_soft_lists' warp instructions sat in these eight
-    // conditionals, at 9-12 of 32 lanes.)
+    // (ncu source view of a branching form, one capacity check per append / push: 36 % of k_soft_lists' warp instructions
+    // sat in its eight conditionals, at 9-12 of 32 lanes.)
     if (n + 4 > out_cap || w->sp + 3 > stack_cap) return -1;
-    {
-        const bool e0 = k0 < inf && l0 < 0, e1 = k1 < inf && l1 < 0, e2 = k2 < inf && l2 < 0, e3 = k3 < inf && l3 < 0;
-        if (e0) out[n] = ~l0;
-        n += e0 ? 1 : 0;
-        if (e1) out[n] = ~l1;
-        n += e1 ? 1 : 0;
-        if (e2) out[n] = ~l2;
-        n += e2 ? 1 : 0;
-        if (e3) out[n] = ~l3;
-        n += e3 ? 1 : 0;
-        w->n = n;
-        const bool i0 = k0 < inf && l0 >= 0, i1 = k1 < inf && l1 >= 0, i2 = k2 < inf && l2 >= 0, i3 = k3 < inf && l3 >= 0;
-        const int nearest = i0 ? l0 : (i1 ? l1 : (i2 ? l2 : (i3 ? l3 : -1)));
-        const bool p3 = i3 && (i0 || i1 || i2), p2 = i2 && (i0 || i1), p1 = i1 && i0;
-        int sp = w->sp;
-        if (p3) stack[sp * stack_stride] = l3;
-        sp += p3 ? 1 : 0;
-        if (p2) stack[sp * stack_stride] = l2;
-        sp += p2 ? 1 : 0;
-        if (p1) stack[sp * stack_stride] = l1;
-        sp += p1 ? 1 : 0;
-        w->sp = sp;
-        if (nearest >= 0) { w->cur = nearest; return 1; }
-        if (sp == 0) return 0;
-        w->sp = sp - 1;
-        w->cur = stack[(sp - 1) * stack_stride];
-        return 1;
-    }
-#endif
-    if (k0 < inf && l0 < 0) { if (n == out_cap) return -1; out[n++] = ~l0; }
-    if (k1 < inf && l1 < 0) { if (n == out_cap) return -1; out[n++] = ~l1; }
-    if (k2 < inf && l2 < 0) { if (n == out_cap) return -1; out[n++] = ~l2; }
-    if (k3 < inf && l3 < 0) { if (n == out_cap) return -1; out[n++] = ~l3; }
+    const bool e0 = k0 < inf && l0 < 0, e1 = k1 < inf && l1 < 0, e2 = k2 < inf && l2 < 0, e3 = k3 < inf && l3 < 0;
+    if (e0) out[n] = ~l0;
+    n += e0 ? 1 : 0;
+    if (e1) out[n] = ~l1;
+    n += e1 ? 1 : 0;
+    if (e2) out[n] = ~l2;
+    n += e2 ? 1 : 0;
+    if (e3) out[n] = ~l3;
+    n += e3 ? 1 : 0;
     w->n = n;
-    int next = -1;                                                        // nearest inner child so far (going far -> near)
-    if (k3 < inf && l3 >= 0) next = l3;
-    if (k2 < inf && l2 >= 0) { if (next >= 0) { if (w->sp == stack_cap) return -1; stack[w->sp * stack_stride] = next; ++w->sp; } next = l2; }
-    if (k1 < inf && l1 >= 0) { if (next >= 0) { if (w->sp == stack_cap) return -1; stack[w->sp * stack_stride] = next; ++w->sp; } next = l1; }
-    if (k0 < inf && l0 >= 0) { if (next >= 0) { if (w->sp == stack_cap) return -1; stack[w->sp * stack_stride] = next; ++w->sp; } next = l0; }
-    if (next >= 0) { w->cur = next; return 1; }
-    if (w->sp == 0) return 0;
-    --w->sp;
-    w->cur = stack[w->sp * stack_stride];
+    const bool i0 = k0 < inf && l0 >= 0, i1 = k1 < inf && l1 >= 0, i2 = k2 < inf && l2 >= 0, i3 = k3 < inf && l3 >= 0;
+    const int nearest = i0 ? l0 : (i1 ? l1 : (i2 ? l2 : (i3 ? l3 : -1)));
+    const bool p3 = i3 && (i0 || i1 || i2), p2 = i2 && (i0 || i1), p1 = i1 && i0;
+    int sp = w->sp;
+    if (p3) stack[sp * stack_stride] = l3;
+    sp += p3 ? 1 : 0;
+    if (p2) stack[sp * stack_stride] = l2;
+    sp += p2 ? 1 : 0;
+    if (p1) stack[sp * stack_stride] = l1;
+    sp += p1 ? 1 : 0;
+    w->sp = sp;
+    if (nearest >= 0) { w->cur = nearest; return 1; }
+    if (sp == 0) return 0;
+    w->sp = sp - 1;
+    w->cur = stack[(sp - 1) * stack_stride];
     return 1;
 }
 

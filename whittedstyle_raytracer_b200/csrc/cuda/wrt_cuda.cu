@@ -46,6 +46,21 @@ struct TimedLaunch {
     bool on_chain;
 };
 
+// Grids and work claiming of the persistent traversal kernels (run_queue, dev_traverse.cuh)
+constexpr int kTraceBlocksPerSm = 10;  // persistent shadow / unfused closest-hit kernels: CTAs per SM
+constexpr int kSideBlocksPerSm = 6;    // persistent shadow kernels on the side stream: CTAs per SM.  6 leave register file
+                                       // for two CTAs of the chain's kernel on every SM, so the chain keeps moving beside a
+                                       // long shadow kernel: 4K soft frame 12.73 -> 12.50 ms (5: 12.40, 7: 12.65, 8: 12.70);
+                                       // hard-shadow, 8K and sphere frames within +-0.5 %
+static_assert(kSideBlocksPerSm <= kTraceBlocksPerSm, "the soft-list scratch is sized for kTraceBlocksPerSm CTAs per SM");
+constexpr int kRefill = 16;            // idle lanes that trigger a refill on deep ray-tree levels
+constexpr int kRefill0 = 32;           // level 0 (coherent primary rays and their shadow rays)
+constexpr int kRefillSoft = 24;        // per-ray soft-shadow kernel
+constexpr int kChunkDiv = 16;          // work claiming: chunks of n/(warps*k) items
+
+// run_queue's `refill_cfg` word: idle lanes per refill | chunk divisor << 8
+constexpr int refill_word(int refill) { return refill | (kChunkDiv << 8); }
+
 } // namespace
 
 struct WrtContext {
@@ -56,7 +71,6 @@ struct WrtContext {
     // (wrt_render_device) is joined to them by two events, nothing else runs on it.
     cudaStream_t chain = nullptr, side = nullptr;
     cudaEvent_t ev_in = nullptr, ev_lvl0 = nullptr, ev_mid = nullptr, ev_side = nullptr, ev_out = nullptr;
-    bool overlap = true;
 
     // scene
     wrt::DevScene ds{};
@@ -79,12 +93,9 @@ struct WrtContext {
     float deep_factor = 0.25f;         // automatic mode: current deep-level capacity factor (grows on overflow)
     float prune_rel = 1e-3f;
     bool kernel_timing = false;
-    int refill = 16;                   // idle lanes that trigger a refill on deep ray-tree levels
-    int refill_soft = 24;
     bool shaft_cull = true;            // soft shadows: answer requests whose light shaft is empty without tracing (shaft_cull.h)
     bool soft_lists = true;            // soft shadows: per-request candidate lists (k_soft_lists + k_soft_list_rays) instead of per-ray walks
     long long list_pool_cap_override = 0;
-    int shaft_cull_max_level = 0;      // deepest ray-tree level whose surface stage runs the shaft test (when lists are on)
     wrt::SoftListBuffers list_bufs[WRT_QUEUES] = {};
     wrt::FastBvhBuilder fbvh;          // WRT_HOST_BVH=1 only: the host's binned-SAH build (development A/B)
     bool host_bvh = false;
@@ -93,19 +104,11 @@ struct WrtContext {
     int ploc_coop_grid = 1;            // co-resident CTAs of k_bvh_ploc
     int fast_depth = 0, build_passes = 0;
     bool unlit_cull = true;            // drop shadow requests of lights whose shading terms are exactly 0 at the point
-    int cache_from_level = 0;          // per-ray soft-shadow kernel: occluder cache (99 = off)
-    int chunk_div = 16;                // work claiming: 0 = one atomic per refill, k = chunks of n/(warps*k) items
-    int refill0 = 32;                  // level 0 (coherent primary rays and their shadow rays)
-    int trace_blocks_per_sm = 10;      // persistent shadow / unfused closest-hit kernels
     bool shade0_separate = true;       // level 0 is shaded by its own launch on the side stream (else inside combine)
     int soft_filter = 2;               // 0: off, 1: prune the deep queues' candidate lists (k_soft_filter), 2: level 0's as well
     int deep_split = 5;                // request queues: level 0 | levels 1..deep_split | deeper.  The shadow kernels of levels
                                        // 1..5 run beside the closest-hit chain of levels 6..8 (4K soft frame: 14.55 ms with one
                                        // deep queue, 14.34 / 14.14 / 14.40 with a split at 4 / 5 / 3; 1/8 share 2.56 -> 2.46 ms)
-    int side_blocks_per_sm = 6;        // persistent shadow kernels on the side stream: CTAs per SM (0 = trace_blocks_per_sm).  6 leave
-                                       // register file for two CTAs of the chain's kernel on every SM, so the chain keeps moving
-                                       // beside a long shadow kernel: 4K soft frame 12.73 -> 12.50 ms (5: 12.40, 7: 12.65, 8: 12.70);
-                                       // hard-shadow, 8K and sphere frames within +-0.5 %
     int fb_split = -1;
     bool small_batch_full_levels = true; // automatic sizing: batches under 1 M slots get full-size deep levels
     long long max_batch = 1ll << 25;   // primary slots per batch (8K = 33.2 M slots fits)
@@ -284,17 +287,14 @@ int ensure_frame_buffers(WrtContext* c, unsigned slots) {
     // ones (origins on the bunny) ~30.
     for (int q = 0; q < WRT_QUEUES; q++) {
         wrt::SoftListBuffers& lb = c->list_bufs[q];
-        // Level-0 requests that survive the shaft test at spawn time have 1-2 candidates, deep-level ones (origins on
-        // the bunny) ~30.  A warp reserves region_per_request entries per request of its chunk; the pool holds that for
-        // half of the queue's capacity (queues run far below capacity; a full pool only means per-ray walks).
-        lb.region_per_request = q == 0 ? 4u : 32u;
+        // pool entries per request of the queue's capacity (queues run far below capacity)
         const unsigned long long per_req = q == 0 ? 4ull : 16ull;
         lb.pool_cap = (unsigned)std::min<unsigned long long>(std::max<unsigned long long>(8ull << 20, per_req * fb.preq_cap[q]), 1ull << 30);
         if (!ds.n_point_lights || ds.shadow_type == 0) lb.pool_cap = 64;
         if (c->list_pool_cap_override > 0) lb.pool_cap = (unsigned)c->list_pool_cap_override;     // tests: force the pool-full path
         const bool lists_possible = ds.n_point_lights && ds.shadow_type != 0;
-        if (frame_alloc(c, &lb.scratch, lists_possible ? (size_t)c->num_sms * c->trace_blocks_per_sm * 128 * WRT_LIST_CAP : 1)) return 1;
-        if (frame_alloc(c, &lb.shafts, lists_possible ? (size_t)c->num_sms * c->trace_blocks_per_sm * 4 * WRT_LISTS_CHUNK * WRT_SHAFT_SLOT : 1)) return 1;
+        if (frame_alloc(c, &lb.scratch, lists_possible ? (size_t)c->num_sms * kTraceBlocksPerSm * 128 * WRT_LIST_CAP : 1)) return 1;
+        if (frame_alloc(c, &lb.shafts, lists_possible ? (size_t)c->num_sms * kTraceBlocksPerSm * 4 * WRT_LISTS_CHUNK * WRT_SHAFT_SLOT : 1)) return 1;
         if (frame_alloc(c, &lb.pool, lb.pool_cap)) return 1;
         if (frame_alloc(c, &lb.ref, lists_possible ? fb.preq_cap[q] : 1)) return 1;
         if (frame_alloc(c, &lb.work, lists_possible ? fb.preq_cap[q] : 1)) return 1;
@@ -354,17 +354,21 @@ size_t stack_bytes(WrtContext* c, int threads) { return (size_t)c->stack_rows * 
 
 float prune_value(const WrtContext* c) { return c->traversal == WRT_TRAVERSAL_PRUNED ? c->prune_rel : -1.f; }
 
+// Whether a frame runs its side-stream work beside the chain.  Kernel timing serialises the frame: every launch on the
+// chain stream.  WRT_TIMING_OVERLAP=1 keeps the two streams and turns the event pairs into a timeline of the frame as it
+// really runs: WRT_TIMING_DUMP prints start and end of every launch.
+bool overlap_streams(const WrtContext* c) { return !c->kernel_timing || getenv("WRT_TIMING_OVERLAP") != nullptr; }
+
 // The shadow kernels of request queue q (0: level 0, 1: levels 1..8 together) on stream `st`.
 int enqueue_shadows(WrtContext* c, cudaStream_t st, int q, int& work_seq) {
     using namespace wrt;
     FrameBuffers& fb = c->fb;
     const DevScene& ds = c->ds;
     const int TB = 128;
-    const bool on_side = st == c->side && c->side_blocks_per_sm > 0;
-    const int trace_grid = grid_for(c, on_side ? std::min(c->side_blocks_per_sm, c->trace_blocks_per_sm) : c->trace_blocks_per_sm), wide_grid = grid_for(c, 8);
+    const int trace_grid = grid_for(c, st == c->side ? kSideBlocksPerSm : kTraceBlocksPerSm), wide_grid = grid_for(c, 8);
     const size_t sb = stack_bytes(c, TB);
     auto work_slot = [&]() { int s = C_WORK + 2 * work_seq; ++work_seq; return s; };
-    const int refill = (q == 0 ? c->refill0 : c->refill) | (c->chunk_div << 8);
+    const int refill = refill_word(q == 0 ? kRefill0 : kRefill);
     if (ds.n_point_lights > 0) {
         if (ds.shadow_type == 0) {
             LaunchScope ls(c, st, F_SHADOW_HARD);
@@ -383,14 +387,13 @@ int enqueue_shadows(WrtContext* c, cudaStream_t st, int q, int& work_seq) {
                 const bool filtered = c->soft_filter >= (q == 0 ? 2 : 1);
                 if (filtered) {                                     // triangle-level pruning of the lists
                     LaunchScope ls(c, st, F_SOFT_FILTER);
-                    k_soft_filter<<<WRT_FILTER_DYNAMIC ? c->filter_grid : wide_grid, TB, 0, st>>>(ds, fb, q, lb, WRT_FILTER_DYNAMIC ? work_slot() : 0);
+                    k_soft_filter<<<c->filter_grid, TB, 0, st>>>(ds, fb, q, lb, work_slot());
                 }
                 LaunchScope ls(c, st, F_SHADOW_SOFT);
                 k_soft_list_rays<<<trace_grid, TB, sb, st>>>(ds, fb, q, work_slot(), c->seed, lb, filtered ? 1 : 0);
             } else {
                 LaunchScope ls(c, st, F_SHADOW_SOFT);
-                k_shadow_soft<<<trace_grid, TB, sb, st>>>(ds, fb, q, work_slot(), c->seed, c->refill_soft | (c->chunk_div << 8),
-                                                          c->cache_from_level <= (q == 0 ? 0 : 1) ? 1 : 0);
+                k_shadow_soft<<<trace_grid, TB, sb, st>>>(ds, fb, q, work_slot(), c->seed, refill_word(kRefillSoft), 1);  // occluder cache on
             }
         }
     }
@@ -408,9 +411,7 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     FrameBuffers& fb = c->fb;
     const DevScene& ds = c->ds;
     cudaStream_t st = c->chain;
-    // (kernel timing serialises the frame: every launch on the chain stream.  WRT_TIMING_OVERLAP=1 keeps the two streams and
-    // turns the event pairs into a timeline of the frame as it really runs: WRT_TIMING_DUMP prints start and end of every launch)
-    const bool overlap = c->overlap && (!c->kernel_timing || getenv("WRT_TIMING_OVERLAP") != nullptr);
+    const bool overlap = overlap_streams(c);
     cudaStream_t ss = overlap ? c->side : st;
     PrimaryGen pg;
     pg.cam = c->cam; pg.tm = c->tilemap(); pg.slot0 = slot0;
@@ -418,7 +419,7 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     int work_seq = 0;
     auto work_slot = [&]() { int s = C_WORK + 2 * work_seq; ++work_seq; return s; };
     const int TB = 128;
-    const int trace_grid = grid_for(c, c->trace_blocks_per_sm), wide_grid = grid_for(c, 8);
+    const int trace_grid = grid_for(c, kTraceBlocksPerSm), wide_grid = grid_for(c, 8);
     const size_t sb = stack_bytes(c, TB);
     const float prune = prune_value(c);
     auto cull_for = [&](int d) {
@@ -430,12 +431,12 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
             // deeper levels (~8 %) k_soft_lists finds the empty ones anyway (an empty list), off the critical
             // closest-hit chain.  Without the list kernels the test runs on every level.
             const bool lists_on = c->soft_lists && !ds.has_light_prims;
-            if (c->shaft_cull && ds.shadow_type != 0 && (d <= c->shaft_cull_max_level || !lists_on)) cull |= WRT_CULL_SHAFT;
+            if (c->shaft_cull && ds.shadow_type != 0 && (d == 0 || !lists_on)) cull |= WRT_CULL_SHAFT;
         }
         return cull;
     };
     auto level_kernels = [&](int d) {
-        const int refill = (d == 0 ? c->refill0 : c->refill) | (c->chunk_div << 8);
+        const int refill = refill_word(d == 0 ? kRefill0 : kRefill);
         {
             LaunchScope ls(c, st, F_TRACE);
             if (d == 0) k_trace_closest<true><<<trace_grid, TB, sb, st>>>(ds, fb, pg, d, n, work_slot(), prune, refill);
@@ -722,23 +723,14 @@ int wrt_create(int device, WrtContext** out) {
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, wrt::k_soft_filter, 128, 0) != cudaSuccess || per_sm < 1) per_sm = 4;
         c->filter_grid = c->num_sms * per_sm;           // one wave: the kernel claims its work dynamically
     }
-    // tuning overrides (development only; defaults are what bench.py measures)
-    if (const char* e = getenv("WRT_REFILL")) c->refill = std::max(1, std::min(32, atoi(e)));
-    if (const char* e = getenv("WRT_REFILL_SOFT")) c->refill_soft = std::max(1, std::min(32, atoi(e)));
-    if (const char* e = getenv("WRT_TRACE_BLOCKS")) c->trace_blocks_per_sm = std::max(1, std::min(32, atoi(e)));
-    if (const char* e = getenv("WRT_OVERLAP")) c->overlap = atoi(e) != 0;
-    if (const char* e = getenv("WRT_CACHE_FROM")) c->cache_from_level = atoi(e);
+    // frame options (defaults are what bench.py measures)
     if (const char* e = getenv("WRT_SHAFT_CULL")) c->shaft_cull = atoi(e) != 0;
     if (const char* e = getenv("WRT_UNLIT_CULL")) c->unlit_cull = atoi(e) != 0;
     if (const char* e = getenv("WRT_SOFT_LISTS")) c->soft_lists = atoi(e) != 0;
     if (const char* e = getenv("WRT_LIST_POOL_CAP")) c->list_pool_cap_override = atoll(e);
-    if (const char* e = getenv("WRT_SHAFT_LEVELS")) c->shaft_cull_max_level = atoi(e);
-    if (const char* e = getenv("WRT_CHUNK_DIV")) c->chunk_div = std::max(0, std::min(255, atoi(e)));
-    if (const char* e = getenv("WRT_REFILL0")) c->refill0 = std::max(1, std::min(32, atoi(e)));
     if (const char* e = getenv("WRT_HOST_BVH")) c->host_bvh = atoi(e) != 0;
     if (const char* e = getenv("WRT_SHADE0_SEPARATE")) c->shade0_separate = atoi(e) != 0;
     if (const char* e = getenv("WRT_SOFT_FILTER")) c->soft_filter = atoi(e);
-    if (const char* e = getenv("WRT_SIDE_BLOCKS")) c->side_blocks_per_sm = std::max(0, std::min(32, atoi(e)));
     if (const char* e = getenv("WRT_DEEP_SPLIT")) c->deep_split = std::max(1, std::min(WRT_MAX_DEPTH - 1, atoi(e)));
     if (const char* e = getenv("WRT_DEEP_FACTOR")) { c->deep_factor = std::max(0.001f, std::min(2.f, (float)atof(e))); c->small_batch_full_levels = false; }
     if (const char* e = getenv("WRT_MAX_BATCH")) c->max_batch = std::max(64ll, (atoll(e) + 31) / 32 * 32);   // tests: force multi-batch frames
@@ -1116,8 +1108,8 @@ int wrt_trace_closest_wavefront(WrtContext* c, const float* orig, const float* d
         CK(cudaMemsetAsync(fb.counters, 0, wrt::C_TOTAL * sizeof(unsigned), st));
         c->launches += 3;
         wrt::k_pack_rays<<<grid_for(c, 4), 256, 0, st>>>(o, d, m, fb.ray_o[level & 1], fb.ray_d[level & 1], fb.counters, level);
-        wrt::k_trace_closest<false><<<grid_for(c, c->trace_blocks_per_sm), 128, stack_bytes(c, 128), st>>>(
-            c->ds, fb, pg, level, 0u, wrt::C_WORK, prune_value(c), c->refill | (c->chunk_div << 8));
+        wrt::k_trace_closest<false><<<grid_for(c, kTraceBlocksPerSm), 128, stack_bytes(c, 128), st>>>(
+            c->ds, fb, pg, level, 0u, wrt::C_WORK, prune_value(c), refill_word(kRefill));
         wrt::k_unpack_hits<<<grid_for(c, 4), 256, 0, st>>>(c->ds, o, d, m, fb.hit, (WrtHit*)c->d_scratch[2] + off);
         CK(cudaGetLastError());
     }
@@ -1200,8 +1192,7 @@ int wrt_shadow_requests_wavefront(WrtContext* c, int queue, int flags, const flo
     if (ensure_frame_buffers(c, std::max(c->batch_slots, 1u << 20))) return 1;
     wrt::FrameBuffers& fb = c->fb;
     // the frame's streams: queues 0 and 1 on the side stream (when the frame overlaps them), queue 2 on the chain
-    const bool overlap = c->overlap && (!c->kernel_timing || getenv("WRT_TIMING_OVERLAP") != nullptr);
-    cudaStream_t st = queue < 2 && overlap ? c->side : c->chain;
+    cudaStream_t st = queue < 2 && overlap_streams(c) ? c->side : c->chain;
     const size_t in_bytes = (size_t)n * sizeof(wrt::ShadowRequestIn);
     if (ensure_scratch(c, 0, in_bytes) || ensure_scratch(c, 1, (size_t)n) || ensure_scratch(c, 2, (size_t)n * sizeof(float))) return 1;
     wrt::ShadowRequestIn* d_in = (wrt::ShadowRequestIn*)c->d_scratch[0];
