@@ -12,6 +12,8 @@
  *                             this query bypasses the strategy interface in the reference
  *   wrt_shadow_directional <- Renderer::getShadowCoeffi(Intersection&, Vector4f&)   include/Renderer.hpp:381-400
  *   wrt_render*            <- Renderer::render()                      include/Renderer.hpp:57-137
+ *                             (wrt_render_gbuffer: also the Intersection, shading normal, Od and shadow coefficients
+ *                              of every eye ray, Renderer.hpp:104-125, :176-184, :283-287)
  *                             (traceRay :151-260, blinnPhongShader :265-341, getAreaLightShadowCoeffi :405-414,
  *                              changeNormalDir :417-474), output = PPMGenerator::rgb as 8-bit
  *   wrt_upload_scene       <- the Scene& / PPMGenerator* the Renderer reads (include/Renderer.hpp:38-49)
@@ -120,6 +122,26 @@ int wrt_render(WrtContext* ctx, uint8_t* rgb_host, WrtStats* stats);
  * nodes is queued on the frame's stream (a batch re-rendered after a queue overflow copies again, over its first
  * attempt); wrt_render and wrt_render_device queue no such copy.  Synchronous. */
 int wrt_render_float(WrtContext* ctx, float* rgb_f_host, uint8_t* rgb_host, WrtStats* stats);
+
+/* Per-pixel surface buffers of the frame's eye rays (host memory, width*height pixels, row-major).  Any plane may be
+ * NULL; a NULL plane costs nothing. */
+typedef struct WrtGBuffer {
+    WrtHit* hit;      /* the eye ray's Intersection (Renderer.hpp:104-125 -> UpdateInter): the record wrt_trace_closest
+                         returns for that ray, the miss record on a miss; a light avatar is a hit */
+    float*  normal;   /* x3: inter.nDir as the shader used it, after changeNormalDir (Renderer.hpp:182-184) */
+    float*  albedo;   /* x3: Od, the material's diffuse colour or the texel (Renderer.hpp:176-180) */
+    float*  shadow;   /* x n_lights: the coefficient blinnPhongShader multiplies for each light: the hard-shadow product,
+                         lit soft-shadow samples / 50, the directional product */
+} WrtGBuffer;
+/* The frame wrt_render renders (the same image, statistics and kernels), and also, per pixel, what its eye ray met.
+ * Pixels that are not shaded (misses, light avatars) read normal = albedo = 0 and -1 for every light.  A shaded pixel
+ * reads -1 for a light whose diffuse and specular factors are exactly 0 when the frame answered it without a coefficient
+ * (WRT_TRAVERSAL_PRUNED with WRT_UNLIT_CULL on, lights 0..31); a soft-shadow request whose shaft to the light is empty
+ * reads exactly 1.  Per batch, two more kernels (after level 0's surface stage, after the combine) fill device staging
+ * that one device-to-host copy per plane moves to pinned memory (a batch re-rendered after a queue overflow exports
+ * again, over its first attempt); the planes are then scattered to pixels.  With tiles only this rank's pixels are
+ * written, in the planes and in rgb_host.  With all planes NULL this is wrt_render.  Synchronous. */
+int wrt_render_gbuffer(WrtContext* ctx, const WrtGBuffer* gb, uint8_t* rgb_host, WrtStats* stats);
 
 /* Asynchronous form on caller-provided device memory and stream (cudaStream_t as void*;
  * NULL is CUDA's legacy default stream, e.g. torch's default current stream).  d_rgb_tiles receives this rank's pixels in tile

@@ -1214,6 +1214,61 @@ __global__ void __launch_bounds__(256) k_unpack_hits(const __grid_constant__ Dev
     }
 }
 
+// ---- per-pixel surface planes of level 0 (wrt_render_gbuffer), into slot-ordered staging of one batch ----
+// k_gbuffer_hit runs right after level 0's k_surface_spawn: level 1's k_trace_closest overwrites fb.hit.  The record is
+// the one k_unpack_hits builds, from the eye ray regenerated as k_trace_closest<true> generated it (a padding slot gets a
+// miss record; it has no pixel).
+__global__ void __launch_bounds__(256) k_gbuffer_hit(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
+                                                     const __grid_constant__ PrimaryGen pg, unsigned n, WrtHit* out) {
+    for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        f3 o, d;
+        unsigned pixel;
+        primary_ray(pg, i, o, d, pixel);
+        const float4 h = fb.hit[i];
+        Closest c;
+        c.t = h.x; c.prim = __float_as_int(h.y); c.u = h.z; c.v = h.w;
+        out[i] = hit_record(s, o, d, c);
+    }
+}
+
+// k_gbuffer_surface runs after k_combine_resolve (level 0's shadow kernels have finished; nothing after surface_warp
+// rewrites a level-0 surface record or coefficient).  A shaded node (surf[4g].w holds a primitive >= 0) exports what
+// surface_warp stored: the shading normal after changeNormalDir, Od, and per light the coefficient blinn_phong
+// multiplies (soft point lights: lit samples / 50, as blinn_phong divides).  A light < 32 whose terms vanish was never
+// given a coefficient when level 0 ran with WRT_CULL_UNLIT: light_terms_vanish on surface_warp's inputs finds it again,
+// and it reads -1.  Unshaded nodes (miss, light avatar, padding): normal and albedo 0, every coefficient -1.
+// NULL planes are skipped.
+__global__ void __launch_bounds__(256) k_gbuffer_surface(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
+                                                         unsigned n, int cull, float* normal, float* albedo, float* shadow) {
+    for (unsigned g = blockIdx.x * blockDim.x + threadIdx.x; g < n; g += gridDim.x * blockDim.x) {
+        const float4* sv = fb.surf + 4 * (size_t)g;
+        const float4 s0 = sv[0];
+        const bool shaded = __float_as_int(s0.w) >= 0;
+        const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
+        const float4 s1 = shaded ? sv[1] : zero, s2 = shaded ? sv[2] : zero;
+        if (normal) { normal[3 * (size_t)g] = s1.x; normal[3 * (size_t)g + 1] = s1.y; normal[3 * (size_t)g + 2] = s1.z; }
+        if (albedo) { albedo[3 * (size_t)g] = s2.x; albedo[3 * (size_t)g + 1] = s2.y; albedo[3 * (size_t)g + 2] = s2.z; }
+        if (!shadow) continue;
+        const f3 pos = mk3(s0), nDir = mk3(s1);
+        const bool unlit_cull = shaded && (cull & WRT_CULL_UNLIT);
+        f3 p_eye_dir = mk3(0.f, 0.f, 0.f);
+        float shade_n = 0.f;
+        if (unlit_cull) {
+            p_eye_dir = normalized(mk3(sv[3]) - pos);
+            shade_n = load_material(s, __float_as_int(s1.w)).n;
+        }
+        for (int li = 0; li < s.n_lights; li++) {
+            const WrtLight* L = s.lights + li;
+            float v = -1.f;
+            if (shaded && !(unlit_cull && li < 32 && light_terms_vanish(L, p_eye_dir, pos, nDir, shade_n))) {
+                v = fb.coeff[(size_t)g * s.n_lights + li];
+                if (float_equal(L->pos[3], 1.f) && s.shadow_type != 0) v = v / (float)WRT_SOFT_SAMPLES;
+            }
+            shadow[(size_t)g * s.n_lights + li] = v;
+        }
+    }
+}
+
 // ---- shadow requests answered by the FRAME's shadow kernels (wrt_shadow_requests_wavefront: the tests put their
 // requests through k_shadow_hard, the candidate-list kernels, k_shadow_soft and k_shadow_directional themselves) ----
 struct ShadowRequestIn {

@@ -61,6 +61,21 @@ constexpr int kChunkDiv = 16;          // work claiming: chunks of n/(warps*k) i
 // run_queue's `refill_cfg` word: idle lanes per refill | chunk divisor << 8
 constexpr int refill_word(int refill) { return refill | (kChunkDiv << 8); }
 
+// Planes a frame can export per batch, in slot order: the level-0 colour {rgb, fr} (wrt_render_float) and the surface
+// planes of wrt_render_gbuffer.  Bit k of WrtContext::exports selects plane k.
+enum ExportPlane { X_FLOAT, X_HIT, X_NORMAL, X_ALBEDO, X_SHADOW, X_PLANES };
+constexpr unsigned X_SURFACE = (1u << X_NORMAL) | (1u << X_ALBEDO) | (1u << X_SHADOW);
+
+// Bytes plane k takes per slot
+size_t plane_bytes(int k, int n_lights) {
+    switch (k) {
+    case X_FLOAT: return sizeof(float4);
+    case X_HIT: return sizeof(WrtHit);
+    case X_NORMAL: case X_ALBEDO: return 3 * sizeof(float);
+    default: return (size_t)n_lights * sizeof(float);
+    }
+}
+
 } // namespace
 
 struct WrtContext {
@@ -127,9 +142,14 @@ struct WrtContext {
     size_t d_image_bytes = 0;
     uint8_t* h_image = nullptr;        // pinned staging
     size_t h_image_bytes = 0;
-    float4* h_float = nullptr;         // pinned, slot order: level-0 {colour, fr} of every local slot (wrt_render_float)
-    size_t h_float_bytes = 0;
-    bool copy_float = false;           // set for the duration of wrt_render_float: each batch copies its level 0 to h_float
+    // Per-batch exports of wrt_render_float / wrt_render_gbuffer, queued on the chain stream behind each batch: `exports`
+    // (X_* bits) is set for the duration of those calls only.  h_plane[k]: pinned, slot order, every local slot;
+    // d_plane[k]: one batch's device staging of the surface planes (X_FLOAT copies fb.node_a itself).
+    unsigned exports = 0;
+    void* h_plane[X_PLANES] = {};
+    size_t h_plane_bytes[X_PLANES] = {};
+    void* d_plane[X_PLANES] = {};
+    size_t d_plane_bytes[X_PLANES] = {};
 
     // batch-query scratch
     void* d_scratch[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};
@@ -306,6 +326,19 @@ int ensure_frame_buffers(WrtContext* c, unsigned slots) {
     return 0;
 }
 
+// Grows a pinned host or device buffer to at least `bytes`; its contents are not kept.
+int ensure_buffer(void** p, size_t* have, size_t bytes, bool pinned) {
+    bytes = std::max<size_t>(bytes, 256);
+    if (*have >= bytes) return 0;
+    if (*p) { if (pinned) cudaFreeHost(*p); else cudaFree(*p); }
+    *p = nullptr;
+    *have = 0;
+    if (pinned) CK(cudaMallocHost(p, bytes));
+    else CK(cudaMalloc(p, bytes));
+    *have = bytes;
+    return 0;
+}
+
 int ensure_scratch(WrtContext* c, int k, size_t bytes) {
     if (c->scratch_bytes[k] >= bytes) return 0;
     if (c->d_scratch[k]) cudaFree(c->d_scratch[k]);
@@ -415,6 +448,10 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     cudaStream_t ss = overlap ? c->side : st;
     PrimaryGen pg;
     pg.cam = c->cam; pg.tm = c->tilemap(); pg.slot0 = slot0;
+    for (int k = X_HIT; k < X_PLANES; k++)             // device staging of the exported surface planes: one batch
+        if ((c->exports >> k & 1u) && ensure_buffer(&c->d_plane[k], &c->d_plane_bytes[k], (size_t)n * plane_bytes(k, ds.n_lights), false))
+            return 1;
+    auto d_plane = [&](int k) { return (c->exports >> k & 1u) ? c->d_plane[k] : nullptr; };
     CK(cudaMemsetAsync(fb.counters, 0, C_TOTAL * sizeof(unsigned), st));
     int work_seq = 0;
     auto work_slot = [&]() { int s = C_WORK + 2 * work_seq; ++work_seq; return s; };
@@ -450,6 +487,10 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
         CK(cudaEventRecord(c->ev_lvl0, st));
         CK(cudaStreamWaitEvent(ss, c->ev_lvl0, 0));
     }
+    if (d_plane(X_HIT)) {                              // before level 1's k_trace_closest overwrites fb.hit
+        ++c->launches;
+        k_gbuffer_hit<<<wide_grid, 256, 0, st>>>(ds, fb, pg, n, (WrtHit*)d_plane(X_HIT));
+    }
     // Level 0's shadow + shade kernels run beside the deep chain on the side stream, then the shadow kernels of levels
     // 1..split (queue 1) as soon as those levels' surface stages are done; the chain goes on with the deeper levels and
     // ends with their shadow kernels (queue 2).  A deep level holds few, long, incoherent rays and leaves most of the SMs
@@ -477,8 +518,18 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
         void* args[] = {(void*)&ds, (void*)&fb, (void*)&tm, (void*)&slot0, (void*)&n, (void*)&shade_from, (void*)&d_image, (void*)&d_packed};
         CK(cudaLaunchCooperativeKernel((const void*)k_combine_resolve, dim3(c->coop_grid), dim3(256), args, 0, st));
     }
-    if (c->copy_float)                                 // the combined level-0 colours this batch quantised, in slot order
-        CK(cudaMemcpyAsync(c->h_float + slot0, fb.node_a, (size_t)n * sizeof(float4), cudaMemcpyDeviceToHost, st));
+    if (c->exports & X_SURFACE) {
+        ++c->launches;
+        k_gbuffer_surface<<<wide_grid, 256, 0, st>>>(ds, fb, n, cull_for(0), (float*)d_plane(X_NORMAL), (float*)d_plane(X_ALBEDO),
+                                                     (float*)d_plane(X_SHADOW));
+    }
+    // this batch's slots of every exported plane; X_FLOAT: the combined level-0 colours this batch quantised
+    for (int k = 0; k < X_PLANES; k++) {
+        if (!(c->exports >> k & 1u)) continue;
+        const size_t b = plane_bytes(k, ds.n_lights);
+        const void* src = k == X_FLOAT ? (const void*)fb.node_a : c->d_plane[k];
+        CK(cudaMemcpyAsync((char*)c->h_plane[k] + (size_t)slot0 * b, src, (size_t)n * b, cudaMemcpyDeviceToHost, st));
+    }
     CK(cudaGetLastError());
     if (C_WORK + 2 * work_seq > C_TOTAL) return fail("internal: work counters exceed the counter block");
     return 0;
@@ -747,7 +798,10 @@ void wrt_destroy(WrtContext* c) {
     for (int k = 0; k < 5; k++) if (c->d_scratch[k]) cudaFree(c->d_scratch[k]);
     if (c->d_image) cudaFree(c->d_image);
     if (c->h_image) cudaFreeHost(c->h_image);
-    if (c->h_float) cudaFreeHost(c->h_float);
+    for (int k = 0; k < X_PLANES; k++) {
+        if (c->h_plane[k]) cudaFreeHost(c->h_plane[k]);
+        if (c->d_plane[k]) cudaFree(c->d_plane[k]);
+    }
     if (c->h_counters) cudaFreeHost(c->h_counters);
     if (c->h_stage) cudaFreeHost(c->h_stage);
     for (cudaEvent_t e : c->event_pool) cudaEventDestroy(e);
@@ -1299,24 +1353,54 @@ int wrt_render_float(WrtContext* c, float* rgb_f_host, uint8_t* rgb_host, WrtSta
     CK(cudaSetDevice(c->device));
     if (!c->has_cam) return fail("wrt_render_float: no camera set");
     const long long slots = c->local_slots(c->rank, c->world);
-    const size_t bytes = (size_t)std::max(slots, 1ll) * sizeof(float4);
-    if (c->h_float_bytes < bytes) {
-        if (c->h_float) cudaFreeHost(c->h_float);
-        c->h_float = nullptr; c->h_float_bytes = 0;
-        CK(cudaMallocHost((void**)&c->h_float, bytes));
-        c->h_float_bytes = bytes;
-    }
-    c->copy_float = true;
+    if (ensure_buffer(&c->h_plane[X_FLOAT], &c->h_plane_bytes[X_FLOAT], (size_t)std::max(slots, 1ll) * sizeof(float4), true)) return 1;
+    c->exports = 1u << X_FLOAT;
     const int rc = wrt_render(c, rgb_host, stats);     // synchronous: every batch's copy has landed when it returns
-    c->copy_float = false;
+    c->exports = 0;
     if (rc) return rc;
+    const float4* h_float = (const float4*)c->h_plane[X_FLOAT];
     wrt::TileMap tm = c->tilemap();
     for (long long s = 0; s < slots; s++) {
         int x, y;
         if (tm.slot_to_pixel(s, c->rank, x, y)) {
             float* p = rgb_f_host + 3 * ((size_t)y * tm.width + x);
-            p[0] = c->h_float[s].x; p[1] = c->h_float[s].y; p[2] = c->h_float[s].z;
+            p[0] = h_float[s].x; p[1] = h_float[s].y; p[2] = h_float[s].z;
         }
+    }
+    return 0;
+}
+
+int wrt_render_gbuffer(WrtContext* c, const WrtGBuffer* gb, uint8_t* rgb_host, WrtStats* stats) {
+    if (!c || !gb || !rgb_host) return fail("wrt_render_gbuffer: null argument");
+    CK(cudaSetDevice(c->device));
+    if (!c->has_scene) return fail("wrt_render_gbuffer: no scene uploaded");
+    if (!c->has_cam) return fail("wrt_render_gbuffer: no camera set");
+    const int nl = c->ds.n_lights;
+    const long long slots = c->local_slots(c->rank, c->world);
+    void* const dst[X_PLANES] = {nullptr, gb->hit, gb->normal, gb->albedo, gb->shadow};
+    unsigned exports = 0;
+    for (int k = X_HIT; k < X_PLANES; k++) {
+        if (!dst[k]) continue;
+        exports |= 1u << k;
+        if (ensure_buffer(&c->h_plane[k], &c->h_plane_bytes[k], (size_t)std::max(slots, 1ll) * plane_bytes(k, nl), true)) return 1;
+    }
+    c->exports = exports;
+    const int rc = wrt_render(c, rgb_host, stats);     // synchronous: every batch's copies have landed when it returns
+    c->exports = 0;
+    if (rc || !exports) return rc;
+    const WrtHit* h_hit = (const WrtHit*)c->h_plane[X_HIT];
+    const float* h_normal = (const float*)c->h_plane[X_NORMAL];
+    const float* h_albedo = (const float*)c->h_plane[X_ALBEDO];
+    const float* h_shadow = (const float*)c->h_plane[X_SHADOW];
+    wrt::TileMap tm = c->tilemap();
+    for (long long s = 0; s < slots; s++) {
+        int x, y;
+        if (!tm.slot_to_pixel(s, c->rank, x, y)) continue;
+        const size_t p = (size_t)y * tm.width + x;
+        if (gb->hit) gb->hit[p] = h_hit[s];
+        if (gb->normal) for (int k = 0; k < 3; k++) gb->normal[3 * p + k] = h_normal[3 * s + k];
+        if (gb->albedo) for (int k = 0; k < 3; k++) gb->albedo[3 * p + k] = h_albedo[3 * s + k];
+        if (gb->shadow) for (int k = 0; k < nl; k++) gb->shadow[(size_t)nl * p + k] = h_shadow[(size_t)nl * s + k];
     }
     return 0;
 }

@@ -207,6 +207,41 @@ class Renderer:
         self.last_stats = stats_dict(st)
         return out_f, out
 
+    GBUFFER_PLANES = ("hit", "normal", "albedo", "shadow")
+
+    def render_gbuffer(self, planes=GBUFFER_PLANES, out: dict | None = None) -> dict:
+        """The frame render() renders, with per-pixel surface buffers of its eye rays (wrt_render_gbuffer).  Returns a
+        dict: "rgb" (H, W, 3) uint8 and each requested plane: "hit" (H, W) cabi.HIT_DTYPE, the eye ray's Intersection;
+        "normal" and "albedo" (H, W, 3) float32, the shading normal and Od (0 where nothing is shaded); "shadow"
+        (H, W, n_lights) float32, the coefficient the shader multiplies for each light (-1 where the frame computed
+        none: unshaded pixels, and lights whose terms vanish in the pruned mode).  `out` may supply any of these arrays;
+        with tiles only this rank's pixels are written."""
+        cam = self.scene.camera
+        h, w = cam.height, cam.width
+        want = {"rgb": ((h, w, 3), np.uint8), "hit": ((h, w), np.dtype(cabi.HIT_DTYPE)),
+                "normal": ((h, w, 3), np.float32), "albedo": ((h, w, 3), np.float32),
+                "shadow": ((h, w, self.scene.desc.n_lights), np.float32)}
+        planes = tuple(planes)
+        unknown = set(planes) - set(self.GBUFFER_PLANES)
+        if unknown:
+            raise ValueError(f"render_gbuffer: unknown planes {sorted(unknown)}; choose from {self.GBUFFER_PLANES}")
+        res = {}
+        gb = cabi.WrtGBuffer()
+        for name in ("rgb",) + planes:
+            shape, dtype = want[name]
+            a = (out or {}).get(name)
+            if a is None:
+                a = np.zeros(shape, dtype)
+            elif a.dtype != dtype or a.shape != shape or not a.flags.c_contiguous:
+                raise ValueError(f"render_gbuffer: out[{name!r}] must be a C-contiguous {shape} {np.dtype(dtype)} array")
+            res[name] = a
+            if name != "rgb":
+                setattr(gb, name, a.ctypes.data)
+        st = cabi.WrtStats()
+        self.ctx._check(self.ctx.lib.wrt_render_gbuffer(self.ctx.h, C.byref(gb), res["rgb"].ctypes.data, C.byref(st)))
+        self.last_stats = stats_dict(st)
+        return res
+
     def render_device(self, d_ptr: int, stream: int | None = None):
         """Asynchronous render of this rank's tiles into device memory (tile order)."""
         self.ctx._check(self.ctx.lib.wrt_render_device(self.ctx.h, d_ptr, stream))
