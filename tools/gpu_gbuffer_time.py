@@ -1,7 +1,7 @@
-"""Cost of the per-pixel surface planes: wrt_render against wrt_render_gbuffer with every plane and with `hit` only, on the
-4K workloads, alternating the three calls round by round.  Host wall time of the synchronous call (output arrays
-allocated once and reused, so no first-touch page faults are timed) and the frame's device time (gpu_ms: first kernel
-to the last batch's copies).  Prints one JSON object with the card's name and power limit.
+"""Cost of the exported planes: wrt_render against wrt_render_float, and against wrt_render_gbuffer with every plane and
+with `hit` only, on the 4K workloads, alternating the four calls round by round.  Host wall time of the synchronous call
+(output arrays allocated once and reused, so no first-touch page faults are timed) and the frame's device time (gpu_ms:
+first kernel to the last batch's copies).  Prints one JSON object with the card's name and power limit.
 Usage: gpu_gbuffer_time.py [--rounds N] [--out FILE] [workload ...]"""
 import argparse
 import json
@@ -11,6 +11,8 @@ import sys
 import tempfile
 import time
 from pathlib import Path
+
+import numpy as np
 
 REPO = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(REPO))
@@ -41,7 +43,9 @@ def main():
         r = Renderer(scene)
         full = r.render_gbuffer()                       # allocates the output arrays once (and warms every mode)
         hit_only = {"rgb": full["rgb"], "hit": full["hit"]}
+        rgb_f = np.zeros(full["rgb"].shape, np.float32)
         calls = {"render": lambda: r.render(out=full["rgb"]),
+                 "render_float": lambda: r.render_float(out_f=rgb_f, out=full["rgb"]),
                  "gbuffer_all": lambda: r.render_gbuffer(out=full),
                  "gbuffer_hit": lambda: r.render_gbuffer(planes=("hit",), out=hit_only)}
         for f in calls.values():

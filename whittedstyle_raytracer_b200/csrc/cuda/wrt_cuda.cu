@@ -121,7 +121,7 @@ struct WrtContext {
     bool unlit_cull = true;            // drop shadow requests of lights whose shading terms are exactly 0 at the point
     bool shade0_separate = true;       // level 0 is shaded by its own launch on the side stream (else inside combine)
     int soft_filter = 2;               // 0: off, 1: prune the deep queues' candidate lists (k_soft_filter), 2: level 0's as well
-    int deep_split = 5;                // request queues: level 0 | levels 1..deep_split | deeper.  The shadow kernels of levels
+    int deep_split = 5;                // request queues: level 0 | levels 1..deep_split (1..8) | deeper.  The shadow kernels of levels
                                        // 1..5 run beside the closest-hit chain of levels 6..8 (4K soft frame: 14.55 ms with one
                                        // deep queue, 14.34 / 14.14 / 14.40 with a split at 4 / 5 / 3; 1/8 share 2.56 -> 2.46 ms)
     int fb_split = -1;
@@ -273,12 +273,10 @@ int ensure_frame_buffers(WrtContext* c, unsigned slots) {
     if (nodes64 > 0x7fffff00ull) return fail("frame batch too large for 32-bit node indices");
     if (nodes64 * std::max(1, ds.n_lights) > 0xffffffffffull) return fail("too many (node, light) pairs");
     fb.cap0 = cap0; fb.capd = capd; fb.n_node_cap = (unsigned)nodes64;
-    const unsigned long long deep_nodes = (unsigned long long)(WRT_MAX_DEPTH - 1) * capd;
     auto req_cap = [](unsigned long long nodes, int lights) {
         return (unsigned)std::min<unsigned long long>(nodes * (unsigned long long)std::max(1, lights), 0xffffff00ull);
     };
-    (void)deep_nodes;
-    const int split = std::max(1, std::min(WRT_MAX_DEPTH - 1, c->deep_split));
+    const int split = c->deep_split;
     const unsigned long long q_nodes[WRT_QUEUES] = {cap0, (unsigned long long)split * capd, (unsigned long long)(WRT_MAX_DEPTH - 1 - split) * capd};
     for (int q = 0; q < WRT_QUEUES; q++) {
         fb.preq_cap[q] = req_cap(std::max(q_nodes[q], 1ull), ds.n_point_lights);
@@ -339,16 +337,6 @@ int ensure_buffer(void** p, size_t* have, size_t bytes, bool pinned) {
     return 0;
 }
 
-int ensure_scratch(WrtContext* c, int k, size_t bytes) {
-    if (c->scratch_bytes[k] >= bytes) return 0;
-    if (c->d_scratch[k]) cudaFree(c->d_scratch[k]);
-    c->d_scratch[k] = nullptr;
-    c->scratch_bytes[k] = 0;
-    CK(cudaMalloc(&c->d_scratch[k], bytes));
-    c->scratch_bytes[k] = bytes;
-    return 0;
-}
-
 cudaEvent_t next_event(WrtContext* c) {
     if (c->event_next == c->event_pool.size()) {
         cudaEvent_t e;
@@ -387,16 +375,41 @@ size_t stack_bytes(WrtContext* c, int threads) { return (size_t)c->stack_rows * 
 
 float prune_value(const WrtContext* c) { return c->traversal == WRT_TRAVERSAL_PRUNED ? c->prune_rel : -1.f; }
 
+// Grows device scratch slot k (0..4) of the batch queries to at least `bytes`
+int grow_scratch(WrtContext* c, int k, size_t bytes) { return ensure_buffer(&c->d_scratch[k], &c->scratch_bytes[k], bytes, false); }
+
+// Grows scratch slot k and queues the copy of the caller's input into it on the chain stream
+int stage_in(WrtContext* c, int k, const void* src, size_t bytes) {
+    if (grow_scratch(c, k, bytes)) return 1;
+    CK(cudaMemcpyAsync(c->d_scratch[k], src, bytes, cudaMemcpyHostToDevice, c->chain));
+    return 0;
+}
+
+// Copies a result from the device to host memory on `st`; returns once it has landed
+int copy_out(cudaStream_t st, void* dst, const void* src, size_t bytes) {
+    CK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return 0;
+}
+
+// One thread per item of a batch query, at most 8 CTAs of 128 threads per SM (the kernels stride over the rest)
+int query_grid(WrtContext* c, int64_t n) { return (int)std::min<int64_t>((n + 127) / 128, grid_for(c, 8)); }
+
 // Whether a frame runs its side-stream work beside the chain.  Kernel timing serialises the frame: every launch on the
 // chain stream.  WRT_TIMING_OVERLAP=1 keeps the two streams and turns the event pairs into a timeline of the frame as it
 // really runs: WRT_TIMING_DUMP prints start and end of every launch.
 bool overlap_streams(const WrtContext* c) { return !c->kernel_timing || getenv("WRT_TIMING_OVERLAP") != nullptr; }
 
-// The shadow kernels of request queue q (0: level 0, 1: levels 1..8 together) on stream `st`.
-int enqueue_shadows(WrtContext* c, cudaStream_t st, int q, int& work_seq) {
+// The stream request queue q's shadow kernels run on: queues 0 and 1 beside the closest-hit chain on the side stream
+// (when the frame overlaps the streams), queue 2 at the end of the chain.
+cudaStream_t queue_stream(const WrtContext* c, int q) { return q < 2 && overlap_streams(c) ? c->side : c->chain; }
+
+// The shadow kernels of request queue q (0: level 0, 1: levels 1..deep_split, 2: deeper) on the queue's stream.
+int enqueue_shadows(WrtContext* c, int q, int& work_seq) {
     using namespace wrt;
     FrameBuffers& fb = c->fb;
     const DevScene& ds = c->ds;
+    const cudaStream_t st = queue_stream(c, q);
     const int TB = 128;
     const int trace_grid = grid_for(c, st == c->side ? kSideBlocksPerSm : kTraceBlocksPerSm), wide_grid = grid_for(c, 8);
     const size_t sb = stack_bytes(c, TB);
@@ -445,7 +458,7 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     const DevScene& ds = c->ds;
     cudaStream_t st = c->chain;
     const bool overlap = overlap_streams(c);
-    cudaStream_t ss = overlap ? c->side : st;
+    cudaStream_t ss = queue_stream(c, 0);               // level 0's shadow + shade work
     PrimaryGen pg;
     pg.cam = c->cam; pg.tm = c->tilemap(); pg.slot0 = slot0;
     for (int k = X_HIT; k < X_PLANES; k++)             // device staging of the exported surface planes: one batch
@@ -495,21 +508,21 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     // 1..split (queue 1) as soon as those levels' surface stages are done; the chain goes on with the deeper levels and
     // ends with their shadow kernels (queue 2).  A deep level holds few, long, incoherent rays and leaves most of the SMs
     // idle, and a persistent traversal kernel ends with its longest ray: the shadow work fills those gaps.
-    if (enqueue_shadows(c, ss, 0, work_seq)) return 1;
+    if (enqueue_shadows(c, 0, work_seq)) return 1;
     if (c->shade0_separate) {
         LaunchScope ls(c, ss, F_SHADE);
         k_shade<<<wide_grid, 256, 0, ss>>>(ds, fb, n, 0, 0);
     }
-    const int split = std::max(1, std::min(WRT_MAX_DEPTH - 1, c->deep_split));
+    const int split = c->deep_split;
     for (int d = 1; d <= split; d++) level_kernels(d);
     if (overlap) {
         CK(cudaEventRecord(c->ev_mid, st));
         CK(cudaStreamWaitEvent(ss, c->ev_mid, 0));
     }
-    if (enqueue_shadows(c, ss, 1, work_seq)) return 1;
+    if (enqueue_shadows(c, 1, work_seq)) return 1;
     if (overlap) CK(cudaEventRecord(c->ev_side, ss));
     for (int d = split + 1; d < WRT_MAX_DEPTH; d++) level_kernels(d);
-    if (split < WRT_MAX_DEPTH - 1 && enqueue_shadows(c, st, 2, work_seq)) return 1;
+    if (split < WRT_MAX_DEPTH - 1 && enqueue_shadows(c, 2, work_seq)) return 1;
     if (overlap) CK(cudaStreamWaitEvent(st, c->ev_side, 0));
     {
         LaunchScope ls(c, st, F_COMBINE);
@@ -592,8 +605,22 @@ bool grow_after_overflow(WrtContext* c) {
     return false;
 }
 
-// Renders the spans on `todo` (popped from the back) synchronously, re-rendering what overflows.
-int render_spans_sync(WrtContext* c, std::vector<std::pair<long long, long long>>& todo, uint8_t* d_image, uint8_t* d_packed) {
+using Spans = std::vector<std::pair<long long, long long>>;    // spans {first slot, slots} of a frame, popped from the back
+
+// The span [s0, s0+n) overflowed a queue: pushes what renders it next onto `todo` — the same span once the deep levels
+// grew, else its two halves.  Automatic sizing remembers the halved batch for the following frames.
+int requeue_overflowed(WrtContext* c, Spans& todo, long long s0, long long n) {
+    if (grow_after_overflow(c)) { todo.push_back({s0, n}); return 0; }
+    if (n <= 64) return fail("ray queue overflow on a 64-slot batch: raise queue_factor");
+    long long half = ((n / 2 + 31) / 32) * 32;
+    if (c->queue_factor <= 0.f) c->learned_batch = std::min(c->learned_batch, half);
+    todo.push_back({s0 + half, n - half});
+    todo.push_back({s0, half});
+    return 0;
+}
+
+// Renders the spans on `todo` synchronously, re-rendering what overflows.
+int render_spans_sync(WrtContext* c, Spans& todo, uint8_t* d_image, uint8_t* d_packed) {
     cudaStream_t st = c->chain;
     while (!todo.empty()) {
         auto [s0, n] = todo.back();
@@ -604,15 +631,10 @@ int render_spans_sync(WrtContext* c, std::vector<std::pair<long long, long long>
         CK(cudaStreamSynchronize(st));
         if (c->h_counters[wrt::C_OVERFLOW]) {
             ++c->stats.overflow_retries;
-            if (grow_after_overflow(c)) { todo.push_back({s0, n}); continue; }
-            if (n <= 64) return fail("ray queue overflow on a 64-slot batch: raise queue_factor");
-            long long half = ((n / 2 + 31) / 32) * 32;
-            if (c->queue_factor <= 0.f) c->learned_batch = std::min(c->learned_batch, half);
-            todo.push_back({s0 + half, n - half});
-            todo.push_back({s0, half});
-            continue;
+            if (requeue_overflowed(c, todo, s0, n)) return 1;
+        } else {
+            add_batch_stats(c, c->h_counters);
         }
-        add_batch_stats(c, c->h_counters);
     }
     return 0;
 }
@@ -648,7 +670,7 @@ int render_all(WrtContext* c, cudaStream_t user, bool join_user, uint8_t* d_imag
         CK(cudaStreamWaitEvent(st, c->ev_in, 0));
     }
     CK(cudaEventRecord(c->ev_begin, st));
-    std::vector<std::pair<long long, long long>> todo;
+    Spans todo;
     for (long long s0 = total; s0 > 0;) {              // push in reverse so spans pop in order
         long long b = (s0 - 1) / max_batch * max_batch;
         todo.push_back({b, s0 - b});
@@ -676,19 +698,12 @@ int finish_frame(WrtContext* c) {
         c->frame_pending = false;
         if (c->h_counters[wrt::C_OVERFLOW]) {
             // the single-batch frame overflowed a queue: redo it synchronously (larger deep levels, or in halves)
-            const long long total = c->local_slots(c->rank, c->world);
             memset(&c->stats, 0, sizeof c->stats);
             c->stats.overflow_retries = 1;
-            std::vector<std::pair<long long, long long>> todo;
-            if (grow_after_overflow(c)) todo.push_back({0, total});
-            else {
-                if (total <= 64) return fail("ray queue overflow on a 64-slot batch: raise queue_factor");
-                long long half = ((total / 2 + 31) / 32) * 32;
-                if (c->queue_factor <= 0.f) c->learned_batch = std::min(c->learned_batch, half);
-                todo.push_back({half, total - half});
-                todo.push_back({0, half});
-            }
-            if (render_spans_sync(c, todo, c->last_image, c->last_packed)) return 1;
+            Spans todo;
+            if (requeue_overflowed(c, todo, 0, c->local_slots(c->rank, c->world)) ||
+                render_spans_sync(c, todo, c->last_image, c->last_packed))
+                return 1;
             CK(cudaEventRecord(c->ev_end, st));
             CK(cudaStreamSynchronize(st));
         } else {
@@ -718,6 +733,86 @@ void tally_kernel_times(WrtContext* c) {
                     tl.on_chain ? "chain" : "side", t0 * 1e3f, t1 * 1e3f);
         }
     }
+}
+
+// Copies a finished frame's row-major 8-bit image to the caller: straight into a page-locked buffer, else through the
+// pinned staging h_image.  With tiles only this rank's pixels are defined: those are copied, the rest of the caller's
+// buffer is left alone.
+int deliver_image(WrtContext* c, const uint8_t* d_image, uint8_t* rgb_host, size_t bytes) {
+    cudaStream_t st = c->chain;
+    cudaPointerAttributes attr;
+    const bool user_pinned = c->world == 1 && cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess &&
+                             attr.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    if (user_pinned) return copy_out(st, rgb_host, d_image, bytes);
+    if (ensure_buffer((void**)&c->h_image, &c->h_image_bytes, bytes, true) || copy_out(st, c->h_image, d_image, bytes)) return 1;
+    if (c->world == 1) memcpy(rgb_host, c->h_image, bytes);
+    else {
+        const wrt::TileMap tm = c->tilemap();
+        const long long slots = c->local_slots(c->rank, c->world);
+        for (long long s = 0; s < slots; s++) {
+            int x, y;
+            if (!tm.slot_to_pixel(s, c->rank, x, y)) continue;
+            const size_t o = 3 * ((size_t)y * tm.width + x);
+            rgb_host[o] = c->h_image[o]; rgb_host[o + 1] = c->h_image[o + 1]; rgb_host[o + 2] = c->h_image[o + 2];
+        }
+    }
+    return 0;
+}
+
+// The frame wrt_render renders, and every plane k whose dst[k] is not NULL (host memory, row-major: rgb of X_FLOAT's
+// {rgb, fr}, the whole slot of the others).  enqueue_batch copies each batch's slots of those planes to pinned
+// h_plane[k]; loops over this rank's slots then scatter them to pixels.  `who` names the caller in error messages.
+int render_exports(WrtContext* c, void* const dst[X_PLANES], uint8_t* rgb_host, WrtStats* stats, const char* who) {
+    CK(cudaSetDevice(c->device));
+    if (!c->has_cam) return fail(std::string(who) + ": no camera set");
+    const int nl = c->ds.n_lights;
+    const long long slots = c->local_slots(c->rank, c->world);
+    unsigned exports = 0;
+    for (int k = 0; k < X_PLANES; k++) {
+        if (!dst[k]) continue;
+        exports |= 1u << k;
+        if (ensure_buffer(&c->h_plane[k], &c->h_plane_bytes[k], (size_t)std::max(slots, 1ll) * plane_bytes(k, nl), true)) return 1;
+    }
+    c->exports = exports;
+    const int rc = wrt_render(c, rgb_host, stats);     // synchronous: every batch's copies have landed when it returns
+    c->exports = 0;
+    if (rc || !exports) return rc;
+    // This scatter is most of the host time of both calls at 4K.  Its loops copy typed, fixed-size values, and the colour
+    // and the surface planes have a loop each, the colour's last: one loop body testing all five planes per pixel, and
+    // the same loops run through a shared walk with a lambda per body, made these calls 1-8 % slower (NVIDIA B200 host,
+    // 1000 W, 4K workloads).
+    const wrt::TileMap tm = c->tilemap();
+    if (exports & ~(1u << X_FLOAT)) {
+        WrtHit* const hit = (WrtHit*)dst[X_HIT];
+        float* const normal = (float*)dst[X_NORMAL];
+        float* const albedo = (float*)dst[X_ALBEDO];
+        float* const shadow = (float*)dst[X_SHADOW];
+        const WrtHit* h_hit = (const WrtHit*)c->h_plane[X_HIT];
+        const float* h_normal = (const float*)c->h_plane[X_NORMAL];
+        const float* h_albedo = (const float*)c->h_plane[X_ALBEDO];
+        const float* h_shadow = (const float*)c->h_plane[X_SHADOW];
+        for (long long s = 0; s < slots; s++) {
+            int x, y;
+            if (!tm.slot_to_pixel(s, c->rank, x, y)) continue;
+            const size_t p = (size_t)y * tm.width + x;
+            if (hit) hit[p] = h_hit[s];
+            if (normal) for (int k = 0; k < 3; k++) normal[3 * p + k] = h_normal[3 * s + k];
+            if (albedo) for (int k = 0; k < 3; k++) albedo[3 * p + k] = h_albedo[3 * s + k];
+            if (shadow) for (int k = 0; k < nl; k++) shadow[(size_t)nl * p + k] = h_shadow[(size_t)nl * s + k];
+        }
+    }
+    if (float* const rgb_f = (float*)dst[X_FLOAT]) {
+        const float4* h_float = (const float4*)c->h_plane[X_FLOAT];
+        for (long long s = 0; s < slots; s++) {
+            int x, y;
+            if (tm.slot_to_pixel(s, c->rank, x, y)) {
+                float* q = rgb_f + 3 * ((size_t)y * tm.width + x);
+                q[0] = h_float[s].x; q[1] = h_float[s].y; q[2] = h_float[s].z;
+            }
+        }
+    }
+    return 0;
 }
 
 } // namespace
@@ -881,12 +976,7 @@ int wrt_upload_scene(WrtContext* c, const WrtSceneDesc* s) {
         total += (p.bytes + 255) & ~(size_t)255;
     }
     total = std::max<size_t>(total, 256);
-    if (c->h_stage_bytes < total) {
-        if (c->h_stage) cudaFreeHost(c->h_stage);
-        c->h_stage = nullptr; c->h_stage_bytes = 0;
-        CK(cudaMallocHost((void**)&c->h_stage, total + total / 4));
-        c->h_stage_bytes = total + total / 4;
-    }
+    if (c->h_stage_bytes < total && ensure_buffer((void**)&c->h_stage, &c->h_stage_bytes, total + total / 4, true)) return 1;
     for (const Part& p : parts) if (p.bytes) memcpy(c->h_stage + p.off, p.src, p.bytes);
     uint8_t* d_stage = nullptr;
     if (dev_alloc(c, total, (void**)&d_stage)) return 1;
@@ -1122,20 +1212,15 @@ static int batch_common(WrtContext* c, int64_t n) {
 int wrt_trace_closest(WrtContext* c, const float* orig, const float* dir, int64_t n, WrtHit* hits) {
     if (batch_common(c, n)) return 1;
     if (n == 0) return 0;
+    const size_t vb = (size_t)n * 3 * sizeof(float), hb = (size_t)n * sizeof(WrtHit);
+    if (stage_in(c, 0, orig, vb) || stage_in(c, 1, dir, vb) || grow_scratch(c, 2, hb)) return 1;
     cudaStream_t st = c->chain;
-    size_t vb = (size_t)n * 3 * sizeof(float);
-    if (ensure_scratch(c, 0, vb) || ensure_scratch(c, 1, vb) || ensure_scratch(c, 2, (size_t)n * sizeof(WrtHit))) return 1;
-    CK(cudaMemcpyAsync(c->d_scratch[0], orig, vb, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(c->d_scratch[1], dir, vb, cudaMemcpyHostToDevice, st));
-    int grid = (int)std::min<int64_t>((n + 127) / 128, grid_for(c, 8));
     ++c->launches;
-    wrt::k_batch_closest<<<grid, 128, stack_bytes(c, 128), st>>>(c->ds, (const float*)c->d_scratch[0],
-                                                                  (const float*)c->d_scratch[1], n,
-                                                                  (WrtHit*)c->d_scratch[2], prune_value(c));
+    wrt::k_batch_closest<<<query_grid(c, n), 128, stack_bytes(c, 128), st>>>(c->ds, (const float*)c->d_scratch[0],
+                                                                              (const float*)c->d_scratch[1], n,
+                                                                              (WrtHit*)c->d_scratch[2], prune_value(c));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(hits, c->d_scratch[2], (size_t)n * sizeof(WrtHit), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    return copy_out(st, hits, c->d_scratch[2], hb);
 }
 
 // The same query through the frame's own deep-level closest-hit kernel: the rays are written into ray-tree level 1's arrays
@@ -1148,10 +1233,8 @@ int wrt_trace_closest_wavefront(WrtContext* c, const float* orig, const float* d
     if (ensure_frame_buffers(c, std::max(c->batch_slots, 1u << 20))) return 1;
     wrt::FrameBuffers& fb = c->fb;
     const int64_t chunk = fb.capd / 2;
-    size_t vb = (size_t)n * 3 * sizeof(float);
-    if (ensure_scratch(c, 0, vb) || ensure_scratch(c, 1, vb) || ensure_scratch(c, 2, (size_t)n * sizeof(WrtHit))) return 1;
-    CK(cudaMemcpyAsync(c->d_scratch[0], orig, vb, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(c->d_scratch[1], dir, vb, cudaMemcpyHostToDevice, st));
+    const size_t vb = (size_t)n * 3 * sizeof(float), hb = (size_t)n * sizeof(WrtHit);
+    if (stage_in(c, 0, orig, vb) || stage_in(c, 1, dir, vb) || grow_scratch(c, 2, hb)) return 1;
     wrt::PrimaryGen pg;
     memset(&pg, 0, sizeof pg);
     const int level = 1;
@@ -1167,32 +1250,25 @@ int wrt_trace_closest_wavefront(WrtContext* c, const float* orig, const float* d
         wrt::k_unpack_hits<<<grid_for(c, 4), 256, 0, st>>>(c->ds, o, d, m, fb.hit, (WrtHit*)c->d_scratch[2] + off);
         CK(cudaGetLastError());
     }
-    CK(cudaMemcpyAsync(hits, c->d_scratch[2], (size_t)n * sizeof(WrtHit), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    return copy_out(st, hits, c->d_scratch[2], hb);
 }
 
 static int batch_shadow(WrtContext* c, const float* pos, const float* ndir, const float* lightpos, int64_t n,
                         float* coeff, int mode) {
     if (batch_common(c, n)) return 1;
     if (n == 0) return 0;
+    const size_t vb = (size_t)n * 3 * sizeof(float);
+    if (stage_in(c, 0, pos, vb) || stage_in(c, 1, ndir, vb) || stage_in(c, 2, lightpos, vb) ||
+        grow_scratch(c, 3, (size_t)n * sizeof(float)))
+        return 1;
     cudaStream_t st = c->chain;
-    size_t vb = (size_t)n * 3 * sizeof(float);
-    for (int k = 0; k < 3; k++) if (ensure_scratch(c, k, std::max(vb, c->scratch_bytes[k]))) return 1;
-    if (ensure_scratch(c, 3, (size_t)n * sizeof(float))) return 1;
-    CK(cudaMemcpyAsync(c->d_scratch[0], pos, vb, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(c->d_scratch[1], ndir, vb, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(c->d_scratch[2], lightpos, vb, cudaMemcpyHostToDevice, st));
-    int grid = (int)std::min<int64_t>((n + 127) / 128, grid_for(c, 8));
     ++c->launches;
-    wrt::k_batch_shadow<<<grid, 128, stack_bytes(c, 128), st>>>(c->ds, (const float*)c->d_scratch[0],
-                                                                 (const float*)c->d_scratch[1],
-                                                                 (const float*)c->d_scratch[2], n,
-                                                                 (float*)c->d_scratch[3], mode, prune_value(c));
+    wrt::k_batch_shadow<<<query_grid(c, n), 128, stack_bytes(c, 128), st>>>(c->ds, (const float*)c->d_scratch[0],
+                                                                             (const float*)c->d_scratch[1],
+                                                                             (const float*)c->d_scratch[2], n,
+                                                                             (float*)c->d_scratch[3], mode, prune_value(c));
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(coeff, c->d_scratch[3], (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    return copy_out(st, coeff, c->d_scratch[3], (size_t)n * sizeof(float));
 }
 
 int wrt_shadow_hard(WrtContext* c, const float* pos, const float* ndir, const float* lightpos, int64_t n, float* coeff) {
@@ -1207,22 +1283,16 @@ int wrt_shadow_directional(WrtContext* c, const float* pos, const int32_t* self_
                            int64_t n, float* coeff) {
     if (batch_common(c, n)) return 1;
     if (n == 0) return 0;
-    cudaStream_t st = c->chain;
-    if (ensure_scratch(c, 0, (size_t)n * 12) || ensure_scratch(c, 1, (size_t)n * 4) ||
-        ensure_scratch(c, 2, (size_t)n * 16) || ensure_scratch(c, 3, (size_t)n * 4))
+    if (stage_in(c, 0, pos, (size_t)n * 12) || stage_in(c, 1, self_object, (size_t)n * 4) ||
+        stage_in(c, 2, lightdir4, (size_t)n * 16) || grow_scratch(c, 3, (size_t)n * 4))
         return 1;
-    CK(cudaMemcpyAsync(c->d_scratch[0], pos, (size_t)n * 12, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(c->d_scratch[1], self_object, (size_t)n * 4, cudaMemcpyHostToDevice, st));
-    CK(cudaMemcpyAsync(c->d_scratch[2], lightdir4, (size_t)n * 16, cudaMemcpyHostToDevice, st));
-    int grid = (int)std::min<int64_t>((n + 127) / 128, grid_for(c, 8));
+    cudaStream_t st = c->chain;
     ++c->launches;
-    wrt::k_batch_shadow_directional<<<grid, 128, stack_bytes(c, 128), st>>>(
+    wrt::k_batch_shadow_directional<<<query_grid(c, n), 128, stack_bytes(c, 128), st>>>(
         c->ds, (const float*)c->d_scratch[0], (const int*)c->d_scratch[1], (const float*)c->d_scratch[2], n,
         (float*)c->d_scratch[3], c->traversal == WRT_TRAVERSAL_EXHAUSTIVE ? 1 : 0);
     CK(cudaGetLastError());
-    CK(cudaMemcpyAsync(coeff, c->d_scratch[3], (size_t)n * 4, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    return 0;
+    return copy_out(st, coeff, c->d_scratch[3], (size_t)n * 4);
 }
 
 // Shadow requests answered by the frame's own shadow kernels: queued into request queue `queue` in input order, exactly as
@@ -1245,10 +1315,9 @@ int wrt_shadow_requests_wavefront(WrtContext* c, int queue, int flags, const flo
     if (c->frame_pending && finish_frame(c)) return 1;
     if (ensure_frame_buffers(c, std::max(c->batch_slots, 1u << 20))) return 1;
     wrt::FrameBuffers& fb = c->fb;
-    // the frame's streams: queues 0 and 1 on the side stream (when the frame overlaps them), queue 2 on the chain
-    cudaStream_t st = queue < 2 && overlap_streams(c) ? c->side : c->chain;
+    cudaStream_t st = queue_stream(c, queue);
     const size_t in_bytes = (size_t)n * sizeof(wrt::ShadowRequestIn);
-    if (ensure_scratch(c, 0, in_bytes) || ensure_scratch(c, 1, (size_t)n) || ensure_scratch(c, 2, (size_t)n * sizeof(float))) return 1;
+    if (grow_scratch(c, 0, in_bytes) || grow_scratch(c, 1, (size_t)n) || grow_scratch(c, 2, (size_t)n * sizeof(float))) return 1;
     wrt::ShadowRequestIn* d_in = (wrt::ShadowRequestIn*)c->d_scratch[0];
     unsigned char* d_kind = (unsigned char*)c->d_scratch[1];
     float* d_out = (float*)c->d_scratch[2];
@@ -1260,12 +1329,10 @@ int wrt_shadow_requests_wavefront(WrtContext* c, int queue, int flags, const flo
     // point or directional light, and the spawn-time shaft test; the host then assigns the queue slots in input order
     CK(cudaMemcpyAsync(d_in, req.data(), in_bytes, cudaMemcpyHostToDevice, st));
     ++c->launches;
-    wrt::k_classify_shadow_requests<<<(int)std::min<int64_t>((n + 127) / 128, grid_for(c, 8)), 128, 0, st>>>(
-        c->ds, d_in, n, (flags & WRT_REQ_SHAFT_CULL) ? 1 : 0, d_kind);
+    wrt::k_classify_shadow_requests<<<query_grid(c, n), 128, 0, st>>>(c->ds, d_in, n, (flags & WRT_REQ_SHAFT_CULL) ? 1 : 0, d_kind);
     CK(cudaGetLastError());
     std::vector<unsigned char> kind((size_t)n);
-    CK(cudaMemcpyAsync(kind.data(), d_kind, (size_t)n, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
+    if (copy_out(st, kind.data(), d_kind, (size_t)n)) return 1;
     // one node per request: a chunk fits the queue, the nodes, and the list kernels' 32-bit ray index (nreq * 50 < 2^32)
     const int64_t chunk = (int64_t)std::min<unsigned long long>(
         {(unsigned long long)fb.preq_cap[queue], (unsigned long long)fb.dreq_cap[queue], (unsigned long long)fb.n_node_cap,
@@ -1284,13 +1351,12 @@ int wrt_shadow_requests_wavefront(WrtContext* c, int queue, int flags, const flo
         ++c->launches;
         wrt::k_pack_shadow_requests<<<grid_for(c, 4), 256, 0, st>>>(c->ds, fb, queue, d_in + off, m, counts[k].first, counts[k].second);
         int work_seq = 0;
-        if (enqueue_shadows(c, st, queue, work_seq)) return 1;
+        if (enqueue_shadows(c, queue, work_seq)) return 1;
         ++c->launches;
         wrt::k_unpack_shadow_requests<<<grid_for(c, 4), 256, 0, st>>>(c->ds, fb, d_in + off, m, d_out + off);
         CK(cudaGetLastError());
     }
-    CK(cudaMemcpyAsync(coeff, d_out, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
+    if (copy_out(st, coeff, d_out, (size_t)n * sizeof(float))) return 1;
     if (c->kernel_timing) tally_kernel_times(c);
     return check_debug_bounds();
 }
@@ -1303,106 +1369,25 @@ int wrt_render(WrtContext* c, uint8_t* rgb_host, WrtStats* stats) {
     if (!c->has_cam) return fail("wrt_render: no camera set");
     size_t bytes = (size_t)c->cam.width * c->cam.height * 3;
     if (bytes == 0) return fail("wrt_render: empty image");
-    if (c->d_image_bytes < bytes) {
-        if (c->d_image) cudaFree(c->d_image);
-        c->d_image = nullptr; c->d_image_bytes = 0;
-        CK(cudaMalloc((void**)&c->d_image, bytes));
-        c->d_image_bytes = bytes;
-    }
-    if (c->h_image_bytes < bytes) {
-        if (c->h_image) cudaFreeHost(c->h_image);
-        c->h_image = nullptr; c->h_image_bytes = 0;
-        CK(cudaMallocHost((void**)&c->h_image, bytes));
-        c->h_image_bytes = bytes;
-    }
-    cudaStream_t st = c->chain;
-    if (c->world > 1) CK(cudaMemsetAsync(c->d_image, 0, bytes, st));
-    if (render_all(c, nullptr, false, c->d_image, nullptr)) return 1;
-    if (finish_frame(c)) return 1;
-    cudaPointerAttributes attr;
-    bool user_pinned = c->world == 1 && cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess &&
-                       attr.type == cudaMemoryTypeHost;
-    cudaGetLastError();
-    if (user_pinned) {                                 // caller's buffer is page-locked: no staging copy
-        CK(cudaMemcpyAsync(rgb_host, c->d_image, bytes, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        if (stats) *stats = c->stats;
-        return 0;
-    }
-    CK(cudaMemcpyAsync(c->h_image, c->d_image, bytes, cudaMemcpyDeviceToHost, st));
-    CK(cudaStreamSynchronize(st));
-    if (c->world == 1) memcpy(rgb_host, c->h_image, bytes);
-    else {
-        // only this rank's pixels are defined; copy them, leave the rest of the caller's buffer alone
-        wrt::TileMap tm = c->tilemap();
-        long long slots = c->local_slots(c->rank, c->world);
-        for (long long s = 0; s < slots; s++) {
-            int x, y;
-            if (tm.slot_to_pixel(s, c->rank, x, y)) {
-                size_t o = 3 * ((size_t)y * tm.width + x);
-                rgb_host[o] = c->h_image[o]; rgb_host[o + 1] = c->h_image[o + 1]; rgb_host[o + 2] = c->h_image[o + 2];
-            }
-        }
-    }
+    if (ensure_buffer((void**)&c->d_image, &c->d_image_bytes, bytes, false)) return 1;
+    if (c->world > 1) CK(cudaMemsetAsync(c->d_image, 0, bytes, c->chain));
+    if (render_all(c, nullptr, false, c->d_image, nullptr) || finish_frame(c) || deliver_image(c, c->d_image, rgb_host, bytes))
+        return 1;
     if (stats) *stats = c->stats;
     return 0;
 }
 
 int wrt_render_float(WrtContext* c, float* rgb_f_host, uint8_t* rgb_host, WrtStats* stats) {
     if (!c || !rgb_f_host || !rgb_host) return fail("wrt_render_float: null argument");
-    CK(cudaSetDevice(c->device));
-    if (!c->has_cam) return fail("wrt_render_float: no camera set");
-    const long long slots = c->local_slots(c->rank, c->world);
-    if (ensure_buffer(&c->h_plane[X_FLOAT], &c->h_plane_bytes[X_FLOAT], (size_t)std::max(slots, 1ll) * sizeof(float4), true)) return 1;
-    c->exports = 1u << X_FLOAT;
-    const int rc = wrt_render(c, rgb_host, stats);     // synchronous: every batch's copy has landed when it returns
-    c->exports = 0;
-    if (rc) return rc;
-    const float4* h_float = (const float4*)c->h_plane[X_FLOAT];
-    wrt::TileMap tm = c->tilemap();
-    for (long long s = 0; s < slots; s++) {
-        int x, y;
-        if (tm.slot_to_pixel(s, c->rank, x, y)) {
-            float* p = rgb_f_host + 3 * ((size_t)y * tm.width + x);
-            p[0] = h_float[s].x; p[1] = h_float[s].y; p[2] = h_float[s].z;
-        }
-    }
-    return 0;
+    void* const dst[X_PLANES] = {rgb_f_host};
+    return render_exports(c, dst, rgb_host, stats, "wrt_render_float");
 }
 
 int wrt_render_gbuffer(WrtContext* c, const WrtGBuffer* gb, uint8_t* rgb_host, WrtStats* stats) {
     if (!c || !gb || !rgb_host) return fail("wrt_render_gbuffer: null argument");
-    CK(cudaSetDevice(c->device));
-    if (!c->has_scene) return fail("wrt_render_gbuffer: no scene uploaded");
-    if (!c->has_cam) return fail("wrt_render_gbuffer: no camera set");
-    const int nl = c->ds.n_lights;
-    const long long slots = c->local_slots(c->rank, c->world);
+    if (!c->has_scene) return fail("wrt_render_gbuffer: no scene uploaded");     // the shadow plane's size is its lights'
     void* const dst[X_PLANES] = {nullptr, gb->hit, gb->normal, gb->albedo, gb->shadow};
-    unsigned exports = 0;
-    for (int k = X_HIT; k < X_PLANES; k++) {
-        if (!dst[k]) continue;
-        exports |= 1u << k;
-        if (ensure_buffer(&c->h_plane[k], &c->h_plane_bytes[k], (size_t)std::max(slots, 1ll) * plane_bytes(k, nl), true)) return 1;
-    }
-    c->exports = exports;
-    const int rc = wrt_render(c, rgb_host, stats);     // synchronous: every batch's copies have landed when it returns
-    c->exports = 0;
-    if (rc || !exports) return rc;
-    const WrtHit* h_hit = (const WrtHit*)c->h_plane[X_HIT];
-    const float* h_normal = (const float*)c->h_plane[X_NORMAL];
-    const float* h_albedo = (const float*)c->h_plane[X_ALBEDO];
-    const float* h_shadow = (const float*)c->h_plane[X_SHADOW];
-    wrt::TileMap tm = c->tilemap();
-    for (long long s = 0; s < slots; s++) {
-        int x, y;
-        if (!tm.slot_to_pixel(s, c->rank, x, y)) continue;
-        const size_t p = (size_t)y * tm.width + x;
-        if (gb->hit) gb->hit[p] = h_hit[s];
-        if (gb->normal) for (int k = 0; k < 3; k++) gb->normal[3 * p + k] = h_normal[3 * s + k];
-        if (gb->albedo) for (int k = 0; k < 3; k++) gb->albedo[3 * p + k] = h_albedo[3 * s + k];
-        if (gb->shadow) for (int k = 0; k < nl; k++) gb->shadow[(size_t)nl * p + k] = h_shadow[(size_t)nl * s + k];
-    }
-    return 0;
+    return render_exports(c, dst, rgb_host, stats, "wrt_render_gbuffer");
 }
 
 int wrt_render_device(WrtContext* c, void* d_rgb_tiles, void* cuda_stream) {
@@ -1458,7 +1443,7 @@ int wrt_measure_fp32_peak(WrtContext* c, float* tflops_fma, float* tflops_mul_ad
     if (!c || !tflops_fma || !tflops_mul_add) return fail("wrt_measure_fp32_peak: null argument");
     CK(cudaSetDevice(c->device));
     cudaStream_t st = c->chain;
-    if (ensure_scratch(c, 4, 256)) return 1;
+    if (grow_scratch(c, 4, 256)) return 1;
     const int iters = 1 << 15, blocks = c->num_sms * 8, threads = 256;
     cudaEvent_t e0, e1;
     CK(cudaEventCreate(&e0));
@@ -1656,24 +1641,12 @@ int wrt_multi_render(WrtMulti* m, uint8_t* rgb_host, WrtStats* stats) {
     const size_t bytes = (size_t)c0->cam.width * c0->cam.height * 3;
     if (bytes == 0) return fail("wrt_multi_render: empty image");
     CK(cudaSetDevice(c0->device));
-    if (c0->d_image_bytes < bytes) {
-        CK(cudaDeviceSynchronize());
-        if (c0->d_image) cudaFree(c0->d_image);
-        c0->d_image = nullptr; c0->d_image_bytes = 0;
-        CK(cudaMalloc((void**)&c0->d_image, bytes));
-        c0->d_image_bytes = bytes;
-    }
+    if (c0->d_image_bytes < bytes) CK(cudaDeviceSynchronize());
+    if (ensure_buffer((void**)&c0->d_image, &c0->d_image_bytes, bytes, false)) return 1;
     const int tw = c0->tile_w, thh = c0->tile_h;
     for (int r = 0; r < n; r++) if (wrt_set_tiles(m->ctx[r], tw, thh, r, n)) return 1;
     const long long stride = c0->local_slots(0, n) * 3;               // rank 0 owns the most tiles
-    if (!m->peer_stores) {
-        if (m->gathered_bytes < (size_t)stride * n) {
-            if (m->d_gathered) cudaFree(m->d_gathered);
-            m->d_gathered = nullptr; m->gathered_bytes = 0;
-            CK(cudaMalloc((void**)&m->d_gathered, (size_t)stride * n));
-            m->gathered_bytes = (size_t)stride * n;
-        }
-    }
+    if (!m->peer_stores && ensure_buffer((void**)&m->d_gathered, &m->gathered_bytes, (size_t)stride * n, false)) return 1;
     uint8_t* d_image0 = c0->d_image;
     int rc = multi_run(m, [&](int r) -> int {
         WrtContext* c = m->ctx[r];
@@ -1682,12 +1655,7 @@ int wrt_multi_render(WrtMulti* m, uint8_t* rgb_host, WrtStats* stats) {
             if (render_all(c, nullptr, false, d_image0, nullptr)) return 1;      // stores cross NVLink from the resolve kernel
             return finish_frame(c);
         }
-        if (m->packed_bytes[r] < (size_t)stride) {
-            if (m->d_packed[r]) cudaFree(m->d_packed[r]);
-            m->d_packed[r] = nullptr; m->packed_bytes[r] = 0;
-            CK(cudaMalloc((void**)&m->d_packed[r], (size_t)stride));
-            m->packed_bytes[r] = (size_t)stride;
-        }
+        if (ensure_buffer((void**)&m->d_packed[r], &m->packed_bytes[r], (size_t)stride, false)) return 1;
         if (render_all(c, nullptr, false, nullptr, m->d_packed[r])) return 1;
         if (finish_frame(c)) return 1;
         CK(cudaMemcpyPeerAsync(m->d_gathered + (size_t)r * stride, m->devices[0], m->d_packed[r], c->device, (size_t)stride, c->chain));
@@ -1697,30 +1665,13 @@ int wrt_multi_render(WrtMulti* m, uint8_t* rgb_host, WrtStats* stats) {
     for (int r = 0; r < n; r++) wrt_set_tiles(m->ctx[r], tw, thh, 0, 1);         // the contexts stay usable on their own
     if (rc) return 1;
     CK(cudaSetDevice(c0->device));
-    cudaStream_t st = c0->chain;
     if (!m->peer_stores) {
         wrt_set_tiles(c0, tw, thh, 0, n);
-        int src = wrt_scatter_tiles(c0, m->d_gathered, n, stride, c0->d_image, (void*)st);
+        int src = wrt_scatter_tiles(c0, m->d_gathered, n, stride, c0->d_image, (void*)c0->chain);
         wrt_set_tiles(c0, tw, thh, 0, 1);
         if (src) return 1;
     }
-    cudaPointerAttributes attr;
-    const bool user_pinned = cudaPointerGetAttributes(&attr, rgb_host) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-    cudaGetLastError();
-    if (user_pinned) {
-        CK(cudaMemcpyAsync(rgb_host, c0->d_image, bytes, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-    } else {
-        if (c0->h_image_bytes < bytes) {
-            if (c0->h_image) cudaFreeHost(c0->h_image);
-            c0->h_image = nullptr; c0->h_image_bytes = 0;
-            CK(cudaMallocHost((void**)&c0->h_image, bytes));
-            c0->h_image_bytes = bytes;
-        }
-        CK(cudaMemcpyAsync(c0->h_image, c0->d_image, bytes, cudaMemcpyDeviceToHost, st));
-        CK(cudaStreamSynchronize(st));
-        memcpy(rgb_host, c0->h_image, bytes);
-    }
+    if (deliver_image(c0, c0->d_image, rgb_host, bytes)) return 1;   // the whole frame: c0 is back to one rank
     if (stats) {
         WrtStats t{};
         for (int r = 0; r < n; r++) {
