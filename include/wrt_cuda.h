@@ -148,9 +148,21 @@ int wrt_render_gbuffer(WrtContext* ctx, const WrtGBuffer* gb, uint8_t* rgb_host,
  * order: wrt_tile_pixel_count(ctx, rank, world) * 3 bytes.  Call wrt_finish_device()
  * before reading statistics. */
 int wrt_render_device(WrtContext* ctx, void* d_rgb_tiles, void* cuda_stream);
+/* The frame wrt_render renders, delivered to device memory of ctx's GPU: width*height pixels, row-major, in the host
+ * forms' per-pixel layouts.  d_planes (itself may be NULL) and each of its members, d_rgb_f (3 floats: what
+ * wrt_render_float returns) and d_rgb (3 bytes: what wrt_render returns) may be NULL, but not all of them; a scene
+ * without lights has no shadow plane (d_planes->shadow is ignored).  Every other pointer must be device or managed memory
+ * of ctx's GPU: host memory, pinned included, is refused before anything is enqueued.  Runs like wrt_render_device on
+ * cuda_stream (NULL: the legacy default stream): a single-batch frame returns once enqueued, a multi-batch frame renders
+ * synchronously here.  Besides the frame's own kernels, per batch, k_gbuffer_hit (hit requested) and k_gbuffer_surface
+ * (any of normal, albedo, shadow, d_rgb_f) store straight into the caller's pixels: no staging and no copy.  With tiles
+ * only this rank's pixels are written, in every output.  Call wrt_finish_device() to complete the frame: an overflowed
+ * frame is re-rendered there into the same buffers. */
+int wrt_render_gbuffer_device(WrtContext* ctx, const WrtGBuffer* d_planes, float* d_rgb_f, uint8_t* d_rgb,
+                              void* cuda_stream);
 /* Waits for the frame.  A frame that overflowed a ray queue is re-rendered inside this call
- * (synchronously, into the same d_rgb_tiles); stats->overflow_retries != 0 then tells the caller
- * to repeat whatever it had already enqueued behind the frame on its stream (e.g. the gather). */
+ * (synchronously, into the same d_rgb_tiles, or wrt_render_gbuffer_device's buffers); stats->overflow_retries != 0 then
+ * tells the caller to repeat whatever it had already enqueued behind the frame on its stream (e.g. the gather). */
 int wrt_finish_device(WrtContext* ctx, WrtStats* stats);
 int wrt_get_stats(WrtContext* ctx, WrtStats* stats);
 

@@ -1,7 +1,10 @@
 """Cost of the exported planes: wrt_render against wrt_render_float, and against wrt_render_gbuffer with every plane and
-with `hit` only, on the 4K workloads, alternating the four calls round by round.  Host wall time of the synchronous call
-(output arrays allocated once and reused, so no first-touch page faults are timed) and the frame's device time (gpu_ms:
-first kernel to the last batch's copies).  Prints one JSON object with the card's name and power limit.
+with `hit` only, on the 4K workloads; and on the device, wrt_render_gbuffer_device with all six outputs (8-bit and float
+colour, hit, normal, albedo, shadow) against wrt_render_device into a tile buffer.  The six calls alternate round by
+round.  Host wall time of the call until its results are final (output arrays and tensors allocated once and reused,
+so no first-touch page faults are timed; the device calls include wrt_finish_device) and the frame's device time
+(gpu_ms: first kernel to the last batch's copies or plane stores).  Prints one JSON object with the card's name and
+power limit.
 Usage: gpu_gbuffer_time.py [--rounds N] [--out FILE] [workload ...]"""
 import argparse
 import json
@@ -13,6 +16,7 @@ import time
 from pathlib import Path
 
 import numpy as np
+import torch
 
 REPO = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(REPO))
@@ -44,10 +48,18 @@ def main():
         full = r.render_gbuffer()                       # allocates the output arrays once (and warms every mode)
         hit_only = {"rgb": full["rgb"], "hit": full["hit"]}
         rgb_f = np.zeros(full["rgb"].shape, np.float32)
+        dev_out = r.render_gbuffer_device()             # preallocated tensors of all six outputs
+        tiles = torch.zeros(r.ctx.tile_pixel_count(0, 1) * 3, dtype=torch.uint8, device="cuda")
+
+        def render_device():
+            r.render_device(tiles.data_ptr(), torch.cuda.current_stream().cuda_stream)
+            r.finish_device()
         calls = {"render": lambda: r.render(out=full["rgb"]),
                  "render_float": lambda: r.render_float(out_f=rgb_f, out=full["rgb"]),
                  "gbuffer_all": lambda: r.render_gbuffer(out=full),
-                 "gbuffer_hit": lambda: r.render_gbuffer(planes=("hit",), out=hit_only)}
+                 "gbuffer_hit": lambda: r.render_gbuffer(planes=("hit",), out=hit_only),
+                 "gbuffer_device_all": lambda: r.render_gbuffer_device(out=dev_out),
+                 "render_device": render_device}
         for f in calls.values():
             f()
         wall = {k: [] for k in calls}

@@ -95,7 +95,7 @@ CUDA_SYMBOLS = [
     "wrt_create", "wrt_destroy", "wrt_last_error", "wrt_upload_scene", "wrt_set_camera", "wrt_set_tiles",
     "wrt_set_options", "wrt_enable_kernel_timing", "wrt_trace_closest", "wrt_trace_closest_wavefront", "wrt_shadow_requests_wavefront",
     "wrt_shadow_hard", "wrt_shadow_soft", "wrt_shadow_directional",
-    "wrt_render", "wrt_render_float", "wrt_render_gbuffer", "wrt_render_device", "wrt_finish_device", "wrt_get_stats", "wrt_tile_pixel_count",
+    "wrt_render", "wrt_render_float", "wrt_render_gbuffer", "wrt_render_gbuffer_device", "wrt_render_device", "wrt_finish_device", "wrt_get_stats", "wrt_tile_pixel_count",
     "wrt_scatter_tiles", "wrt_kernel_launch_count", "wrt_get_kernel_times", "wrt_get_kernel_launches", "wrt_measure_fp32_peak",
     "wrt_multi_create", "wrt_multi_destroy", "wrt_multi_device_count", "wrt_multi_context", "wrt_multi_uses_peer_stores",
     "wrt_multi_upload_scene", "wrt_multi_set_camera", "wrt_multi_set_options", "wrt_multi_render",
@@ -166,6 +166,7 @@ def load_cuda() -> C.CDLL:
         lib.wrt_render.argtypes = [vp, vp, C.POINTER(WrtStats)]
         lib.wrt_render_float.argtypes = [vp, vp, vp, C.POINTER(WrtStats)]
         lib.wrt_render_gbuffer.argtypes = [vp, C.POINTER(WrtGBuffer), vp, C.POINTER(WrtStats)]
+        lib.wrt_render_gbuffer_device.argtypes = [vp, C.POINTER(WrtGBuffer), vp, vp, vp]
         lib.wrt_render_device.argtypes = [vp, vp, vp]
         lib.wrt_finish_device.argtypes = [vp, C.POINTER(WrtStats)]
         lib.wrt_get_stats.argtypes = [vp, C.POINTER(WrtStats)]

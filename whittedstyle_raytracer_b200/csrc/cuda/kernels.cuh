@@ -1214,20 +1214,26 @@ __global__ void __launch_bounds__(256) k_unpack_hits(const __grid_constant__ Dev
     }
 }
 
-// ---- per-pixel surface planes of level 0 (wrt_render_gbuffer), into slot-ordered staging of one batch ----
+// ---- per-pixel surface planes of level 0 (wrt_render_gbuffer, wrt_render_gbuffer_device) ----
+// Two output modes.  row_major == 0: slot i of the batch goes to element i of one batch's slot-ordered staging (the host
+// form scatters it to pixels).  row_major != 0: it goes to its pixel y * W + x of the caller's row-major W x H plane
+// (PrimaryGen::tm, slot0: the batch's tile map); padding slots have no pixel and are skipped.
 // k_gbuffer_hit runs right after level 0's k_surface_spawn: level 1's k_trace_closest overwrites fb.hit.  The record is
 // the one k_unpack_hits builds, from the eye ray regenerated as k_trace_closest<true> generated it (a padding slot gets a
-// miss record; it has no pixel).
+// miss record in slot order; it has no pixel).
 __global__ void __launch_bounds__(256) k_gbuffer_hit(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
-                                                     const __grid_constant__ PrimaryGen pg, unsigned n, WrtHit* out) {
+                                                     const __grid_constant__ PrimaryGen pg, unsigned n, int row_major, WrtHit* out) {
     for (unsigned i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
         f3 o, d;
         unsigned pixel;
-        primary_ray(pg, i, o, d, pixel);
+        const bool live = primary_ray(pg, i, o, d, pixel);
+        if (row_major && !live) continue;
         const float4 h = fb.hit[i];
         Closest c;
         c.t = h.x; c.prim = __float_as_int(h.y); c.u = h.z; c.v = h.w;
-        out[i] = hit_record(s, o, d, c);
+        const WrtHit rec = hit_record(s, o, d, c);
+        if (!row_major) out[i] = rec;
+        else if (WRT_IN_BOUNDS(pixel, (size_t)pg.cam.width * pg.cam.height)) out[pixel] = rec;
     }
 }
 
@@ -1237,17 +1243,30 @@ __global__ void __launch_bounds__(256) k_gbuffer_hit(const __grid_constant__ Dev
 // multiplies (soft point lights: lit samples / 50, as blinn_phong divides).  A light < 32 whose terms vanish was never
 // given a coefficient when level 0 ran with WRT_CULL_UNLIT: light_terms_vanish on surface_warp's inputs finds it again,
 // and it reads -1.  Unshaded nodes (miss, light avatar, padding): normal and albedo 0, every coefficient -1.
+// rgb_f (row-major mode only): the combined level-0 colour k_combine_resolve quantised, fb.node_a[g].xyz.
 // NULL planes are skipped.
 __global__ void __launch_bounds__(256) k_gbuffer_surface(const __grid_constant__ DevScene s, const __grid_constant__ FrameBuffers fb,
-                                                         unsigned n, int cull, float* normal, float* albedo, float* shadow) {
+                                                         const __grid_constant__ TileMap tm, long long slot0, unsigned n, int cull,
+                                                         int row_major, float* normal, float* albedo, float* shadow, float* rgb_f) {
     for (unsigned g = blockIdx.x * blockDim.x + threadIdx.x; g < n; g += gridDim.x * blockDim.x) {
+        size_t p = g;                                  // the output element of this node
+        if (row_major) {
+            int x, y;
+            if (!tm.slot_to_pixel(slot0 + g, tm.rank, x, y)) continue;
+            p = (size_t)y * tm.width + x;
+            if (!WRT_IN_BOUNDS(p, (size_t)tm.width * tm.height)) continue;
+        }
+        if (rgb_f) {
+            const float4 c = fb.node_a[g];
+            rgb_f[3 * p] = c.x; rgb_f[3 * p + 1] = c.y; rgb_f[3 * p + 2] = c.z;
+        }
         const float4* sv = fb.surf + 4 * (size_t)g;
         const float4 s0 = sv[0];
         const bool shaded = __float_as_int(s0.w) >= 0;
         const float4 zero = make_float4(0.f, 0.f, 0.f, 0.f);
         const float4 s1 = shaded ? sv[1] : zero, s2 = shaded ? sv[2] : zero;
-        if (normal) { normal[3 * (size_t)g] = s1.x; normal[3 * (size_t)g + 1] = s1.y; normal[3 * (size_t)g + 2] = s1.z; }
-        if (albedo) { albedo[3 * (size_t)g] = s2.x; albedo[3 * (size_t)g + 1] = s2.y; albedo[3 * (size_t)g + 2] = s2.z; }
+        if (normal) { normal[3 * p] = s1.x; normal[3 * p + 1] = s1.y; normal[3 * p + 2] = s1.z; }
+        if (albedo) { albedo[3 * p] = s2.x; albedo[3 * p + 1] = s2.y; albedo[3 * p + 2] = s2.z; }
         if (!shadow) continue;
         const f3 pos = mk3(s0), nDir = mk3(s1);
         const bool unlit_cull = shaded && (cull & WRT_CULL_UNLIT);
@@ -1264,7 +1283,7 @@ __global__ void __launch_bounds__(256) k_gbuffer_surface(const __grid_constant__
                 v = fb.coeff[(size_t)g * s.n_lights + li];
                 if (float_equal(L->pos[3], 1.f) && s.shadow_type != 0) v = v / (float)WRT_SOFT_SAMPLES;
             }
-            shadow[(size_t)g * s.n_lights + li] = v;
+            shadow[p * s.n_lights + li] = v;
         }
     }
 }

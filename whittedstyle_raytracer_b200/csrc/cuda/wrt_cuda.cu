@@ -171,6 +171,8 @@ struct WrtContext {
     bool user_stream_joined = false;
     uint8_t* last_image = nullptr;     // targets of the frame in flight (needed again if an overflowed batch is redone)
     uint8_t* last_packed = nullptr;
+    void* last_planes[X_PLANES] = {};  // wrt_render_gbuffer_device: the frame's row-major device destinations (X_* order,
+                                       // NULL: not requested), released when the frame finishes
     bool frame_pending = false;
     bool has_frame = false;
 
@@ -464,7 +466,11 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     for (int k = X_HIT; k < X_PLANES; k++)             // device staging of the exported surface planes: one batch
         if ((c->exports >> k & 1u) && ensure_buffer(&c->d_plane[k], &c->d_plane_bytes[k], (size_t)n * plane_bytes(k, ds.n_lights), false))
             return 1;
-    auto d_plane = [&](int k) { return (c->exports >> k & 1u) ? c->d_plane[k] : nullptr; };
+    // Host exports (c->exports) go to one batch's slot-ordered staging; the device form's planes (c->last_planes) straight
+    // to their pixels.  A frame has one or the other.
+    void* const* dev = c->last_planes;
+    const int row_major = c->exports ? 0 : 1;
+    auto d_plane = [&](int k) { return (c->exports >> k & 1u) ? c->d_plane[k] : dev[k]; };
     CK(cudaMemsetAsync(fb.counters, 0, C_TOTAL * sizeof(unsigned), st));
     int work_seq = 0;
     auto work_slot = [&]() { int s = C_WORK + 2 * work_seq; ++work_seq; return s; };
@@ -502,7 +508,7 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
     }
     if (d_plane(X_HIT)) {                              // before level 1's k_trace_closest overwrites fb.hit
         ++c->launches;
-        k_gbuffer_hit<<<wide_grid, 256, 0, st>>>(ds, fb, pg, n, (WrtHit*)d_plane(X_HIT));
+        k_gbuffer_hit<<<wide_grid, 256, 0, st>>>(ds, fb, pg, n, row_major, (WrtHit*)d_plane(X_HIT));
     }
     // Level 0's shadow + shade kernels run beside the deep chain on the side stream, then the shadow kernels of levels
     // 1..split (queue 1) as soon as those levels' surface stages are done; the chain goes on with the deeper levels and
@@ -531,10 +537,10 @@ int enqueue_batch(WrtContext* c, long long slot0, unsigned n, uint8_t* d_image, 
         void* args[] = {(void*)&ds, (void*)&fb, (void*)&tm, (void*)&slot0, (void*)&n, (void*)&shade_from, (void*)&d_image, (void*)&d_packed};
         CK(cudaLaunchCooperativeKernel((const void*)k_combine_resolve, dim3(c->coop_grid), dim3(256), args, 0, st));
     }
-    if (c->exports & X_SURFACE) {
+    if ((c->exports & X_SURFACE) || dev[X_FLOAT] || dev[X_NORMAL] || dev[X_ALBEDO] || dev[X_SHADOW]) {
         ++c->launches;
-        k_gbuffer_surface<<<wide_grid, 256, 0, st>>>(ds, fb, n, cull_for(0), (float*)d_plane(X_NORMAL), (float*)d_plane(X_ALBEDO),
-                                                     (float*)d_plane(X_SHADOW));
+        k_gbuffer_surface<<<wide_grid, 256, 0, st>>>(ds, fb, pg.tm, slot0, n, cull_for(0), row_major, (float*)d_plane(X_NORMAL),
+                                                     (float*)d_plane(X_ALBEDO), (float*)d_plane(X_SHADOW), (float*)dev[X_FLOAT]);
     }
     // this batch's slots of every exported plane; X_FLOAT: the combined level-0 colours this batch quantised
     for (int k = 0; k < X_PLANES; k++) {
@@ -640,8 +646,10 @@ int render_spans_sync(WrtContext* c, Spans& todo, uint8_t* d_image, uint8_t* d_p
 }
 
 // Renders all local slots.  A single-batch frame (the common case) is enqueued without any host synchronisation;
-// overflow is checked — and the frame redone — in finish_frame.
-int render_all(WrtContext* c, cudaStream_t user, bool join_user, uint8_t* d_image, uint8_t* d_packed) {
+// overflow is checked — and the frame redone — in finish_frame.  d_planes: wrt_render_gbuffer_device's row-major device
+// planes (X_* order), or NULL.
+int render_all(WrtContext* c, cudaStream_t user, bool join_user, uint8_t* d_image, uint8_t* d_packed,
+               void* const* d_planes = nullptr) {
     if (!c->has_scene) return fail("wrt_render: no scene uploaded");
     if (!c->has_cam) return fail("wrt_render: no camera set");
     if (c->cam.width <= 0 || c->cam.height <= 0) return fail("wrt_render: empty image");
@@ -659,6 +667,7 @@ int render_all(WrtContext* c, cudaStream_t user, bool join_user, uint8_t* d_imag
     c->user_stream = user;
     c->user_stream_joined = join_user;
     c->last_image = d_image; c->last_packed = d_packed;
+    for (int k = 0; k < X_PLANES; k++) c->last_planes[k] = d_planes ? d_planes[k] : nullptr;
     c->has_frame = true;
     cudaStream_t st = c->chain;
     if (total > 0) {
@@ -710,6 +719,7 @@ int finish_frame(WrtContext* c) {
             add_batch_stats(c, c->h_counters);
         }
     }
+    for (void*& p : c->last_planes) p = nullptr;
     if (check_debug_bounds()) return 1;
     float ms = 0.f;
     if (cudaEventElapsedTime(&ms, c->ev_begin, c->ev_end) == cudaSuccess) c->stats.gpu_ms = ms;
@@ -1395,6 +1405,35 @@ int wrt_render_device(WrtContext* c, void* d_rgb_tiles, void* cuda_stream) {
     CK(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)cuda_stream;        // NULL = the legacy default stream, as in CUDA
     return render_all(c, st, true, nullptr, (uint8_t*)d_rgb_tiles);
+}
+
+int wrt_render_gbuffer_device(WrtContext* c, const WrtGBuffer* d_planes, float* d_rgb_f, uint8_t* d_rgb, void* cuda_stream) {
+    const char* who = "wrt_render_gbuffer_device";
+    if (!c) return fail(std::string(who) + ": null context");
+    CK(cudaSetDevice(c->device));
+    if (!c->has_scene) return fail(std::string(who) + ": no scene uploaded");
+    if (!c->has_cam) return fail(std::string(who) + ": no camera set");
+    const WrtGBuffer none{};
+    const WrtGBuffer& gb = d_planes ? *d_planes : none;
+    // a scene without lights has a zero-width shadow plane: not requested
+    void* const dst[X_PLANES] = {d_rgb_f, gb.hit, gb.normal, gb.albedo, c->ds.n_lights > 0 ? gb.shadow : nullptr};
+    const char* const names[X_PLANES] = {"d_rgb_f", "d_planes->hit", "d_planes->normal", "d_planes->albedo", "d_planes->shadow"};
+    if (!d_rgb && std::none_of(dst, dst + X_PLANES, [](void* p) { return p != nullptr; }))
+        return fail(std::string(who) + ": every output is NULL");
+    // every destination is device (or managed) memory of this context's GPU; nothing is enqueued otherwise
+    auto on_device = [&](const void* p, const char* name) {
+        cudaPointerAttributes a;
+        const bool ok = cudaPointerGetAttributes(&a, p) == cudaSuccess &&
+                        (a.type == cudaMemoryTypeDevice || a.type == cudaMemoryTypeManaged) && a.device == c->device;
+        cudaGetLastError();
+        if (!ok) fail(std::string(who) + ": " + name + " is not device memory of device " + std::to_string(c->device) +
+                      " (host memory, pinned included, is refused)");
+        return ok;
+    };
+    if (d_rgb && !on_device(d_rgb, "d_rgb")) return 1;
+    for (int k = 0; k < X_PLANES; k++)
+        if (dst[k] && !on_device(dst[k], names[k])) return 1;
+    return render_all(c, (cudaStream_t)cuda_stream, true, d_rgb, nullptr, dst);
 }
 
 int wrt_finish_device(WrtContext* c, WrtStats* stats) {

@@ -54,6 +54,7 @@ class Context:
         self.lib = cabi.load_cuda()
         self.h = C.c_void_p()
         self._check(self.lib.wrt_create(device, C.byref(self.h)))
+        self.device = device
         self.scene = None
 
     def _check(self, rc):
@@ -240,6 +241,49 @@ class Renderer:
         st = cabi.WrtStats()
         self.ctx._check(self.ctx.lib.wrt_render_gbuffer(self.ctx.h, C.byref(gb), res["rgb"].ctypes.data, C.byref(st)))
         self.last_stats = stats_dict(st)
+        return res
+
+    GBUFFER_DEVICE_PLANES = ("rgb", "rgb_f", "hit", "normal", "albedo", "shadow")
+
+    def render_gbuffer_device(self, planes=GBUFFER_DEVICE_PLANES, out: dict | None = None) -> dict:
+        """The frame render() renders, delivered as CUDA tensors on the context's GPU (wrt_render_gbuffer_device): no pixel
+        crosses to the host.  Returns a dict of the requested planes: "rgb" (H, W, 3) uint8, render()'s image; "rgb_f"
+        (H, W, 3) float32, render_float()'s colour; "hit" (H, W, 15) int32 whose bytes are WrtHit records:
+        `t.cpu().numpy().view(cabi.HIT_DTYPE)[..., 0]` equals render_gbuffer()'s "hit" array; "normal" and "albedo"
+        (H, W, 3) float32 and "shadow" (H, W, n_lights) float32, as render_gbuffer() returns them.  `out` may supply any of
+        these tensors (contiguous, on the context's device, of that dtype and shape); the others are new torch.zeros.  With
+        tiles only this rank's pixels are written.  The frame is enqueued on torch's current stream for the device and
+        finished (finish_device(), which sets last_stats) before this returns; asynchronous use goes through the C ABI,
+        as with render_device()."""
+        import torch
+        cam = self.scene.camera
+        h, w = cam.height, cam.width
+        want = {"rgb": ((h, w, 3), torch.uint8), "rgb_f": ((h, w, 3), torch.float32), "hit": ((h, w, 15), torch.int32),
+                "normal": ((h, w, 3), torch.float32), "albedo": ((h, w, 3), torch.float32),
+                "shadow": ((h, w, self.scene.desc.n_lights), torch.float32)}
+        planes = tuple(planes)
+        if not planes:
+            raise ValueError("render_gbuffer_device: no planes requested")
+        unknown = set(planes) - set(self.GBUFFER_DEVICE_PLANES)
+        if unknown:
+            raise ValueError(f"render_gbuffer_device: unknown planes {sorted(unknown)}; choose from {self.GBUFFER_DEVICE_PLANES}")
+        dev = torch.device("cuda", self.ctx.device)
+        res = {}
+        for name in planes:
+            shape, dtype = want[name]
+            t = (out or {}).get(name)
+            if t is None:
+                t = torch.zeros(shape, dtype=dtype, device=dev)
+            elif (not isinstance(t, torch.Tensor) or t.device != dev or t.dtype != dtype or tuple(t.shape) != shape
+                  or not t.is_contiguous()):
+                raise ValueError(f"render_gbuffer_device: out[{name!r}] must be a contiguous {shape} {dtype} tensor on {dev}")
+            res[name] = t
+        ptr = {k: (t.data_ptr() if t.numel() else None) for k, t in res.items()}
+        gb = cabi.WrtGBuffer(hit=ptr.get("hit"), normal=ptr.get("normal"), albedo=ptr.get("albedo"), shadow=ptr.get("shadow"))
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        self.ctx._check(self.ctx.lib.wrt_render_gbuffer_device(self.ctx.h, C.byref(gb), ptr.get("rgb_f"), ptr.get("rgb"),
+                                                                stream))
+        self.finish_device()
         return res
 
     def render_device(self, d_ptr: int, stream: int | None = None):
